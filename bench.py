@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, one process per GPU)
     python bench.py --impl reference --steps K --warmup W    # reference arm: the reference's own CPU code on host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/*.npy
 
 One bench "step" = one full greedy-Q rollout of a batch: reset + T = 2N env steps for B episodes, each env step being one
 MPNN Q-evaluation + argmax + one fused env-step kernel.  Headline workload = the configuration BASELINE.json's `metric` is
@@ -367,11 +368,17 @@ def headline_config(world):
             "parallelism": "episodes sharded over %d GPU(s), no collective during rollout, all_gather of best cuts" % world}
 
 
+def dump_outputs(out_dir, arrays):
+    """out_dir/<name>.npy for each device tensor of `arrays`, as float64 (exact for the int32 / int8 results), so that
+    the outputs of two builds can be compared array for array."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
-    import __graft_entry__ as ge
-    ge.build()
     import eco_dqn_b200.engine as engine
     from eco_dqn_b200 import _lib
     import ctypes as C
@@ -412,12 +419,13 @@ def run_ours(args):
             self.used_impl = "tcgen05" if (impl != _lib.MPNN_SIMT and self.w.c.packed and self.gs.pm1_only) else "simt"
 
         def step(self, n_steps=None):
+            """-> results() of the rollout: best cut [B], best spins [B, n], steps taken [B]."""
             self.env.reset(spins=self.spins, graph_idx=self.gidx)
             self.env.rollout(self.w, n_steps=n_steps)
-            bc, _, _ = self.env.results()
+            res = self.env.results()
             if self.gathered is not None:
-                dist.all_gather(self.gathered, bc)             # the path's only collective: final best cuts
-            return bc
+                dist.all_gather(self.gathered, res[0])         # the path's only collective: final best cuts
+            return res
 
         def timed(self, warmup, steps, n_steps=None, sample_clocks=False):
             """-> dict(ms_total over `steps` rollouts (max over ranks), mpnn / env kernel averages, launches)."""
@@ -433,7 +441,7 @@ def run_ours(args):
             barrier()
             ev0.record()
             for _ in range(steps):
-                bc = self.step(n_steps)
+                res = self.step(n_steps)
             ev1.record()
             barrier()
             clocks = sampler.stop() if sampler else None
@@ -449,8 +457,8 @@ def run_ours(args):
             if one_launch:                      # per step: forward + argmax + env step inside the resident kernel
                 mpnn_ms, mpnn_n, env_ms, env_n = roll_ms, roll_n, 0.0, 0
             return {"ms_total": float(ms.item()), "mpnn_ms": mpnn_ms / max(mpnn_n, 1), "mpnn_n": mpnn_n,
-                    "env_ms": env_ms / max(env_n, 1), "env_n": env_n, "launches": launches, "clocks": clocks, "best": bc,
-                    "one_launch": one_launch}
+                    "env_ms": env_ms / max(env_n, 1), "env_n": env_n, "launches": launches, "clocks": clocks, "best": res[0],
+                    "results": res, "one_launch": one_launch}
 
         def side_block(self, name, r, steps, env_steps_per_rollout, ranks=1):
             """ms per [MPNN + env step], env-steps/s, roofline fraction of the MPNN forward of this size."""
@@ -474,6 +482,8 @@ def run_ours(args):
     r = head.timed(args.warmup, args.steps, sample_clocks=True)
     ms_total, bc = r["ms_total"], r["best"]
     value = world * B * T * args.steps / (ms_total / 1000.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("best_cut", "best_spins", "steps"), r["results"])))
 
     # ---- the env-step kernel alone at the bench's batch (the rollout applies the step inside the MPNN kernel) ----
     env_small = None
@@ -646,7 +656,15 @@ def main():
     ap.add_argument("--skip-env-only", action="store_true")
     ap.add_argument("--skip-dqn", action="store_true")
     ap.add_argument("--skip-sizes", action="store_true", help="omit the side blocks c1 .. c4")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline workload returned on rank 0 (best_cut [B], "
+                         "best_spins [B, N], steps [B]; 6.6 MB) as DIR/<name>.npy in float64; the inputs are seeded, so "
+                         "two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the CUDA arm (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:
