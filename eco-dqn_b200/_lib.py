@@ -45,6 +45,18 @@ class Env(C.Structure):
                 ("xn", vp), ("xg", vp), ("frac_tab", vp)]
 
 
+class WGraphs(C.Structure):
+    _fields_ = [("G", i32), ("N", i32), ("NP", i32), ("reserved", i32),
+                ("J", vp), ("Jf", vp), ("gscal", vp), ("deg", vp), ("gstat", vp), ("dmax", vp)]
+
+
+class WEnv(C.Structure):
+    _fields_ = [("base", Env), ("h", vp), ("cut", vp)]
+
+
+WGRAPH_NO_DEGREE, WGRAPH_ASYMMETRIC, WGRAPH_NONFINITE = 2, 4, 8   # eco_wgraphs_t.gstat flags
+
+
 class Mpnn(C.Structure):
     _fields_ = [("w_init", vp), ("w_edge", vp), ("w_edge_feat", vp), ("w_msg", vp * 3), ("w_upd", vp * 3),
                 ("w_pool", vp), ("w_read", vp), ("b_read", vp), ("packed", vp)]
@@ -104,6 +116,16 @@ def lib():
         "eco_mpnn_pack": (C.c_int, [P(Mpnn), vp, vp]),
         "eco_mpnn_forward": (C.c_int, [P(Graphs), P(Mpnn), i32, vp, vp, vp, C.c_float, vp, vp, vp, i32, vp]),
         "eco_rollout": (C.c_int, [P(Graphs), P(Env), P(Mpnn), i32, i32, C.c_float, vp, vp, i32, vp, vp, vp, vp]),
+        "eco_wgraphs_workspace_bytes": (C.c_size_t, [i32, i32]),
+        "eco_wgraphs_bind": (C.c_int, [P(WGraphs), vp, i32, i32]),
+        "eco_wgraphs_load_dev": (C.c_int, [P(WGraphs), vp, vp]),
+        "eco_wenv_workspace_bytes": (C.c_size_t, [i32, i32, i32]),
+        "eco_wenv_bind": (C.c_int, [P(WEnv), vp, i32, i32, i32, C.c_double]),
+        "eco_wenv_reset": (C.c_int, [P(WGraphs), P(WEnv), vp, vp, vp]),
+        "eco_wenv_step": (C.c_int, [P(WGraphs), P(WEnv), i32, vp, vp, vp, vp, vp, vp, vp]),
+        "eco_wmpnn_forward": (C.c_int, [P(WGraphs), P(Mpnn), i32, vp, vp, vp, C.c_float, vp, vp, vp, i32, vp]),
+        "eco_wrollout": (C.c_int, [P(WGraphs), P(WEnv), P(Mpnn), i32, i32, C.c_float, vp, vp, i32, vp, vp, vp, vp]),
+        "eco_wenv_results": (C.c_int, [P(WEnv), vp, vp, vp, vp]),
         "eco_session_create": (C.c_int, [P(vp), i32, i32, i32, i32, C.c_double, P(vp), i32]),
         "eco_session_destroy": (None, [vp]),
         "eco_session_rollout": (C.c_int, [vp, vp, vp, vp, i32, C.c_float, vp, vp, vp]),
@@ -121,7 +143,9 @@ EXPORTED = ["eco_last_error", "eco_abi_version", "eco_launch_count", "eco_profil
             "eco_env_bind", "eco_env_set_tables", "eco_env_reset", "eco_env_step", "eco_env_observation",
             "eco_env_best_spins", "eco_env_masked_argmax", "eco_env_results", "eco_graph_aggregate", "eco_mpnn_grad_scratch_bytes", "eco_mpnn_grad", "eco_mpnn_grad_ev", "eco_mpnn_adam", "eco_mpnn_adam_dev", "eco_dp_create", "eco_dp_handle", "eco_dp_open", "eco_dp_adam", "eco_dp_destroy", "eco_mpnn_scratch_bytes", "eco_mpnn_packed_bytes",
             "eco_mpnn_pack", "eco_mpnn_forward", "eco_rollout", "eco_session_create", "eco_session_destroy",
-            "eco_session_rollout"]
+            "eco_session_rollout", "eco_wgraphs_workspace_bytes", "eco_wgraphs_bind", "eco_wgraphs_load_dev",
+            "eco_wenv_workspace_bytes", "eco_wenv_bind", "eco_wenv_reset", "eco_wenv_step", "eco_wmpnn_forward", "eco_wrollout",
+            "eco_wenv_results"]
 
 
 def check(rc):

@@ -158,6 +158,9 @@ class DQN:
         n, T, E = self.n_spins, self.max_steps, self.n_envs
         self._ring_size = int(np.ceil(replay_buffer_size / T)) + 2 * E + 2
         first = [self._new_graph() for _ in range(E)]
+        if not all(engine.is_int8_graph(g) for g in first):
+            raise NotImplementedError("DQN training with real-valued couplings (EdgeType.RANDOM) is not supported: the "
+                                      "training kernels take integer couplings; weighted graphs run rollouts only")
         ring = np.zeros((self._ring_size, n, n), dtype=np.int8)
         ring[:] = engine.graphs_to_int8(first[0])[0]          # placeholder so that every slot holds a valid graph
         self._graphs = engine.GraphSet(ring, device=self.device, min_cut=self.min_cut)

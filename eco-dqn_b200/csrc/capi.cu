@@ -107,6 +107,23 @@ static void carve_env(eco_env_t* e, Carver& c, int B, int N, int T, double basin
     e->frac_tab = c.take<float>((size_t)N + 1);
 }
 
+static void carve_wgraphs(eco_wgraphs_t* g, Carver& c, int G, int N) {
+    const int NP = padded_n(N);
+    g->G = G; g->N = N; g->NP = NP; g->reserved = 0;
+    g->J = c.take<double>((size_t)G * NP * NP);
+    g->Jf = c.take<float>((size_t)G * NP * NP);
+    g->gscal = c.take<double>((size_t)G * 4);
+    g->deg = c.take<float>((size_t)G * NP);
+    g->gstat = c.take<int32_t>((size_t)G * 4);
+    g->dmax = c.take<float>(64);
+}
+
+static void carve_wenv(eco_wenv_t* e, Carver& c, int B, int N, int T, double basin) {
+    carve_env(&e->base, c, B, N, T, basin);
+    e->h = c.take<double>((size_t)B * e->base.NP);
+    e->cut = c.take<double>((size_t)B * 2);
+}
+
 static bool shape_ok(int N) { return N >= 1 && N <= ECO_MAX_SPINS; }
 
 __global__ void frac_tab_kernel(float* tab, int N) {
@@ -475,6 +492,122 @@ int eco_rollout(const eco_graphs_t* g, eco_env_t* env, const eco_mpnn_t* w, int3
         if (rc) return rc;
     }
     return ECO_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ weighted graphs
+size_t eco_wgraphs_workspace_bytes(int32_t G, int32_t N) {
+    if (G < 1 || !shape_ok(N)) return 0;
+    eco_wgraphs_t g;
+    Carver c(nullptr);
+    carve_wgraphs(&g, c, G, N);
+    return c.off;
+}
+
+int eco_wgraphs_bind(eco_wgraphs_t* g, void* ws, int32_t G, int32_t N) {
+    ECO_CHECK_ARG(g && ws, ECO_ERR_INVALID, "eco_wgraphs_bind: null argument");
+    ECO_CHECK_ARG(G >= 1 && shape_ok(N), ECO_ERR_INVALID, "eco_wgraphs_bind: need G >= 1 and 1 <= N <= %d (got G=%d N=%d)",
+                  ECO_MAX_SPINS, G, N);
+    ECO_CHECK_ARG(((uintptr_t)ws & 255) == 0, ECO_ERR_INVALID, "eco_wgraphs_bind: workspace must be 256-byte aligned");
+    Carver c(ws);
+    carve_wgraphs(g, c, G, N);
+    return ECO_OK;
+}
+
+int eco_wgraphs_load_dev(eco_wgraphs_t* g, const double* J_dev, void* stream) {
+    ECO_CHECK_ARG(g && J_dev && g->J, ECO_ERR_INVALID, "eco_wgraphs_load_dev: null argument");
+    ECO_CHECK_ARG(g->reserved == 0, ECO_ERR_UNSUPPORTED, "eco_wgraphs_load_dev: weighted graph sets support OptimisationTarget.CUT only");
+    return launch_wgraph_prepare(g, J_dev, (cudaStream_t)stream);
+}
+
+size_t eco_wenv_workspace_bytes(int32_t B, int32_t N, int32_t T) {
+    if (B < 1 || !shape_ok(N) || T < 1 || T > 65535) return 0;
+    eco_wenv_t e;
+    Carver c(nullptr);
+    carve_wenv(&e, c, B, N, T, 1.0);
+    return c.off;
+}
+
+int eco_wenv_bind(eco_wenv_t* env, void* ws, int32_t B, int32_t N, int32_t T, double basin_reward) {
+    ECO_CHECK_ARG(env && ws, ECO_ERR_INVALID, "eco_wenv_bind: null argument");
+    ECO_CHECK_ARG(B >= 1 && shape_ok(N), ECO_ERR_INVALID, "eco_wenv_bind: need B >= 1 and 1 <= N <= %d", ECO_MAX_SPINS);
+    ECO_CHECK_ARG(T >= 1 && T <= 65535, ECO_ERR_INVALID, "eco_wenv_bind: max_steps must be in [1, 65535] (got %d)", T);
+    ECO_CHECK_ARG(((uintptr_t)ws & 255) == 0, ECO_ERR_INVALID, "eco_wenv_bind: workspace must be 256-byte aligned");
+    Carver c(ws);
+    carve_wenv(env, c, B, N, T, basin_reward);
+    return ECO_OK;
+}
+
+static int check_wpair(const eco_wgraphs_t* g, const eco_wenv_t* env, const char* who) {
+    ECO_CHECK_ARG(g && env, ECO_ERR_INVALID, "%s: null argument", who);
+    ECO_CHECK_ARG(g->N == env->base.N && g->NP == env->base.NP, ECO_ERR_INVALID, "%s: graph set has N=%d but env has N=%d",
+                  who, g->N, env->base.N);
+    ECO_CHECK_ARG(env->base.reserved == 0 && g->reserved == 0, ECO_ERR_UNSUPPORTED,
+                  "%s: weighted graphs support the ECO-DQN configuration only (CUT target, BLS reward, reversible spins)", who);
+    return ECO_OK;
+}
+
+int eco_wenv_reset(const eco_wgraphs_t* g, eco_wenv_t* env, const int32_t* gidx, const int8_t* spins, void* stream) {
+    int rc = check_wpair(g, env, "eco_wenv_reset");
+    if (rc) return rc;
+    ECO_CHECK_ARG(gidx && spins, ECO_ERR_INVALID, "eco_wenv_reset: null argument");
+    return launch_wenv_reset(g, env, gidx, spins, (cudaStream_t)stream);
+}
+
+int eco_wenv_step(const eco_wgraphs_t* g, eco_wenv_t* env, int32_t policy, const int32_t* actions, double* reward,
+                  uint8_t* done, int32_t* ha, double* hr, double* hs, void* stream) {
+    int rc = check_wpair(g, env, "eco_wenv_step");
+    if (rc) return rc;
+    ECO_CHECK_ARG(policy == ECO_POLICY_ACTIONS || policy == ECO_POLICY_GREEDY, ECO_ERR_INVALID,
+                  "eco_wenv_step: policy must be ECO_POLICY_ACTIONS or ECO_POLICY_GREEDY");
+    ECO_CHECK_ARG(policy != ECO_POLICY_ACTIONS || actions, ECO_ERR_INVALID, "eco_wenv_step: actions_dev is NULL");
+    return launch_wenv_step(g, env, policy, actions, reward, done, ha, hr, hs, (cudaStream_t)stream);
+}
+
+int eco_wmpnn_forward(const eco_wgraphs_t* g, const eco_mpnn_t* w, int32_t B, const int32_t* gidx, const float* xn,
+                      const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, int32_t impl,
+                      void* stream) {
+    ECO_CHECK_ARG(g && gidx && xn && xg && scratch, ECO_ERR_INVALID, "eco_wmpnn_forward: null argument");
+    ECO_CHECK_ARG(B >= 1, ECO_ERR_INVALID, "eco_wmpnn_forward: B must be >= 1");
+    int rc = check_weights(w, "eco_wmpnn_forward");
+    if (rc) return rc;
+    // the tensor-core kernels factor the edge stage into contractions with J and |J| in {-1,0,1} (DESIGN.md section 4.2);
+    // a real a_ij does not factor that way
+    ECO_CHECK_ARG(impl != ECO_MPNN_TCGEN05, ECO_ERR_UNSUPPORTED,
+                  "eco_wmpnn_forward: the tensor-core MPNN needs couplings in {-1,0,1}; weighted graphs run on ECO_MPNN_SIMT");
+    ECO_CHECK_ARG(impl == ECO_MPNN_AUTO || impl == ECO_MPNN_SIMT, ECO_ERR_INVALID, "eco_wmpnn_forward: unknown impl %d", impl);
+    return launch_mpnn_simt_w(g, w, B, gidx, xn, xg, norm_max, q, actions, scratch, (cudaStream_t)stream);
+}
+
+int eco_wrollout(const eco_wgraphs_t* g, eco_wenv_t* env, const eco_mpnn_t* w, int32_t n_steps, int32_t policy,
+                 float norm_max, int32_t* act, void* scratch, int32_t impl, int32_t* ha, double* hr, double* hs,
+                 void* stream) {
+    int rc = check_wpair(g, env, "eco_wrollout");
+    if (rc) return rc;
+    ECO_CHECK_ARG(n_steps >= 0, ECO_ERR_INVALID, "eco_wrollout: n_steps < 0");
+    ECO_CHECK_ARG(policy == ECO_POLICY_NETWORK || policy == ECO_POLICY_GREEDY, ECO_ERR_INVALID,
+                  "eco_wrollout: policy must be ECO_POLICY_NETWORK or ECO_POLICY_GREEDY");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (policy == ECO_POLICY_GREEDY) {
+        for (int t = 0; t < n_steps; ++t) {
+            rc = launch_wenv_step(g, env, ECO_POLICY_GREEDY, nullptr, nullptr, nullptr, ha, hr, hs, st);
+            if (rc) return rc;
+        }
+        return ECO_OK;
+    }
+    ECO_CHECK_ARG(act && scratch, ECO_ERR_INVALID, "eco_wrollout: network policy needs actions and mpnn scratch buffers");
+    for (int t = 0; t < n_steps; ++t) {
+        rc = eco_wmpnn_forward(g, w, env->base.B, env->base.graph_idx, env->base.xn, env->base.xg, norm_max, nullptr, act,
+                               scratch, impl, stream);
+        if (rc) return rc;
+        rc = launch_wenv_step(g, env, ECO_POLICY_ACTIONS, act, nullptr, nullptr, ha, hr, hs, st);
+        if (rc) return rc;
+    }
+    return ECO_OK;
+}
+
+int eco_wenv_results(const eco_wenv_t* env, double* best_cut, int8_t* best_spins, int32_t* steps, void* stream) {
+    ECO_CHECK_ARG(env, ECO_ERR_INVALID, "eco_wenv_results: null argument");
+    return launch_wenv_results(env, best_cut, best_spins, steps, (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------------------------------------ session

@@ -124,6 +124,13 @@ int launch_masked_argmax(const eco_env_t* env, const float* q, int32_t* actions,
 int launch_env_results(const eco_env_t* env, int32_t* best_cut, int8_t* best_spins, int32_t* steps, cudaStream_t st);
 int launch_mpnn_simt(const eco_graphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
                      const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);
+int launch_wgraph_prepare(const eco_wgraphs_t* g, const double* dense, cudaStream_t st);
+int launch_wenv_reset(const eco_wgraphs_t* g, eco_wenv_t* we, const int32_t* gidx, const int8_t* spins, cudaStream_t st);
+int launch_wenv_step(const eco_wgraphs_t* g, eco_wenv_t* we, int policy, const int32_t* actions, double* reward, uint8_t* done,
+                     int32_t* ha, double* hr, double* hs, cudaStream_t st);
+int launch_wenv_results(const eco_wenv_t* we, double* best_cut, int8_t* best_spins, int32_t* steps, cudaStream_t st);
+int launch_mpnn_simt_w(const eco_wgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
+                       const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);
 size_t mpnn_simt_scratch_bytes(int B, int N);
 int launch_mpnn_tc(const eco_graphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
                    const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);

@@ -60,6 +60,46 @@ __device__ __forceinline__ int sx16(uint32_t w, int hh) {
 }
 __device__ __forceinline__ int zx16(uint32_t w, int hh) { return (int)prmt(w, 0, (2 * hh) | ((2 * hh + 1) << 4) | 0x4400); }
 
+// The scalar part of one ECO-DQN step (lane 0 of an episode), in the reference's fp64 operation order (appendix A.2):
+// score / normalised score (spinsystem.py:399-400), BLS reward (:418-424), basin reward through the visited set (:443-457),
+// best tracking (:459-463).  delta / delta_n: the score mask and normalised score mask at the action (:393-394).  The
+// visited-set slot `tv` at `slot` of `tab` was requested by the caller (k0 / k1: the Zobrist key after the flip).  Shared
+// by the int8 kernel below and the fp64-field kernel of weighted graphs (weighted.cu).
+struct StepScalars {
+    double score, nscore, best_score, best_nscore, rew;
+    int n_visited;
+    bool new_best;
+};
+__device__ __forceinline__ StepScalars bls_step_scalars(const eco_env_t& env, const double (&sc)[4], double delta,
+                                                        double delta_n, int nimp, int n_visited, uint64_t* tab, uint32_t slot,
+                                                        ulonglong2 tv, uint64_t k0, uint64_t k1) {
+    StepScalars r;
+    r.score = __dadd_rn(sc[0], delta);                                 // :399
+    r.nscore = __dadd_rn(sc[1], delta_n);                              // :400
+    r.rew = 0.0;
+    if (r.score > sc[2]) r.rew = __dsub_rn(r.nscore, sc[3]);           // :418-424
+    if (env.use_basin) {                                               // :443-457
+        const uint64_t w0 = k0 ^ VISITED_SALT0, w1 = k1 ^ VISITED_SALT1;
+        bool is_new = false;
+        for (int probe = 0; probe < env.HCAP; ++probe) {
+            if (tv.x == 0 && tv.y == 0) {
+                *reinterpret_cast<ulonglong2*>(tab + 2 * slot) = make_ulonglong2(w0, w1);
+                is_new = true; ++n_visited;
+                break;
+            }
+            if (tv.x == w0 && tv.y == w1) break;
+            slot = (slot + 1) & (env.HCAP - 1);
+            tv = *reinterpret_cast<const ulonglong2*>(tab + 2 * slot);
+        }
+        if (nimp == 0 && is_new) r.rew = __dadd_rn(r.rew, env.basin_reward);
+    }
+    r.n_visited = n_visited;
+    r.new_best = r.score > sc[2];                                      // :459-463
+    r.best_score = r.new_best ? r.score : sc[2];
+    r.best_nscore = r.new_best ? r.nscore : sc[3];
+    return r;
+}
+
 // Latency-optimised form for NP <= 256: everything that does not depend on the action is requested first, the flipped
 // vertex's old spin / field come from a shuffle, the visited-set slot is prefetched, observable row 1 and the normalised
 // score change come from per-graph tables.  All TPE lanes of the group must call it (group shuffles); lanes of an episode
@@ -207,32 +247,13 @@ __device__ __forceinline__ void env_step_group(const eco_graphs_t& g, const eco_
     int new_best = 0;
     if (lane == 0 && active) {
         if (!use_tab) delta_n = __ddiv_rn((double)delta, qn);           // :394
-        const double score = __dadd_rn(sc[0], (double)delta);           // :399
-        const double nscore = __dadd_rn(sc[1], delta_n);                // :400
-        const double best_score = sc[2], best_nscore = sc[3];
         const int cut = e0.y + delta;
-        double rew = 0.0;
-        if (score > best_score) rew = __dsub_rn(nscore, best_nscore);   // :418-424
-        int n_visited = e1.z;
-        if (env.use_basin) {                                            // :443-457
-            const uint64_t w0 = k0 ^ VISITED_SALT0, w1 = k1 ^ VISITED_SALT1;
-            bool is_new = false;
-            for (int probe = 0; probe < env.HCAP; ++probe) {
-                if (tv.x == 0 && tv.y == 0) {
-                    *reinterpret_cast<ulonglong2*>(tab + 2 * slot) = make_ulonglong2(w0, w1);
-                    is_new = true; ++n_visited;
-                    break;
-                }
-                if (tv.x == w0 && tv.y == w1) break;
-                slot = (slot + 1) & (env.HCAP - 1);
-                tv = *reinterpret_cast<const ulonglong2*>(tab + 2 * slot);
-            }
-            if (nimp == 0 && is_new) rew = __dadd_rn(rew, env.basin_reward);
-        }
+        const StepScalars r = bls_step_scalars(env, sc, (double)delta, delta_n, nimp, e1.z, tab, slot, tv, k0, k1);
+        const double score = r.score, nscore = r.nscore, rew = r.rew, nbs = r.best_score, nbn = r.best_nscore;
+        const int n_visited = r.n_visited;
         int dist = e0.w + (((old_word >> (a & 31)) & 1u) ? -1 : 1);
         int best_cut = e0.z;
-        double nbs = best_score, nbn = best_nscore;
-        if (score > best_score) { nbs = score; nbn = nscore; best_cut = cut; dist = 0; new_best = 1; }   // :459-463
+        if (r.new_best) { best_cut = cut; dist = 0; new_best = 1; }
         const int done = step_new == env.T;                             // :541-544
         int4* epw = reinterpret_cast<int4*>(ep);
         epw[0] = make_int4(step_new, cut, best_cut, dist);

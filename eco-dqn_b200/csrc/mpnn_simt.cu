@@ -1,5 +1,6 @@
 // Kernel family 2a: MPNN Q-network forward + argmax on CUDA cores (fp32).  General path: any int8
-// couplings, any N <= ECO_MAX_SPINS.  Also the on-device cross-check for the tcgen05 kernel (mpnn_tc.cu).
+// couplings, any N <= ECO_MAX_SPINS, and the fp32 couplings of weighted graph sets (eco_wgraphs_t.Jf: the same kernel
+// instantiated on float rows).  Also the on-device cross-check for the tcgen05 kernel (mpnn_tc.cu).
 //
 // Replaces (reference, file:line)
 //   src/networks/mpnn.py:40-77    MPNN.forward
@@ -11,8 +12,8 @@
 //   experiments/utils.py:57-66    argmax action selection (first maximal index)
 //
 // One persistent CTA (8 warps) walks over episodes.  Per episode the node embeddings live in a per-CTA
-// global scratch (L2 resident); neighbour aggregation scans the int8 adjacency row 16 bytes per lane and
-// visits only non-zeros; the 64x64 / 64x128 linears run on 8-vertex tiles per warp (16 accumulators per lane,
+// global scratch (L2 resident); neighbour aggregation scans the adjacency row 16 entries per lane (one 16-byte load
+// for int8, four float4 loads for fp32) and visits only non-zeros; the 64x64 / 64x128 linears run on 8-vertex tiles per warp (16 accumulators per lane,
 // weights transposed in shared memory, inputs broadcast from shared memory).
 #include "eco_common.cuh"
 
@@ -44,12 +45,45 @@ __global__ void transpose_weights_kernel(const eco_mpnn_t w, float* __restrict__
     }
 }
 
+// The graph as the kernel reads it: int8 couplings (eco_graphs_t) or fp32 ones (eco_wgraphs_t.Jf).  V is the type a
+// coupling is handled in (int for int8, so the integer instantiation is the original kernel).
+template <class T>
+struct GView {
+    const T* J;
+    const float* deg;
+    const int32_t* gstat;
+    const float* dmax;
+    int N, NP;
+};
+template <class T> struct CouplingVal { using type = int; };
+template <> struct CouplingVal<float> { using type = float; };
+
+// K consecutive couplings of a row, widened to V: 16 / 8 int8 (one 16- / 8-byte load) or 4 fp32 (one float4 -- wider
+// chunks of fp32 rows push the kernel over its 128-register budget)
+__device__ __forceinline__ void load_row(const int8_t* p, int (&v)[16]) {
+    union { uint4 q; int8_t b[16]; } u;
+    u.q = *reinterpret_cast<const uint4*>(p);
+#pragma unroll
+    for (int k = 0; k < 16; ++k) v[k] = u.b[k];
+}
+__device__ __forceinline__ void load_row(const int8_t* p, int (&v)[8]) {
+    union { uint2 q; int8_t b[8]; } u;
+    u.q = *reinterpret_cast<const uint2*>(p);
+#pragma unroll
+    for (int k = 0; k < 8; ++k) v[k] = u.b[k];
+}
+__device__ __forceinline__ void load_row(const float* p, float (&v)[4]) {
+    const float4 f = *reinterpret_cast<const float4*>(p);
+    v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w;
+}
+
+template <class T>
 struct Smem {
     float wa[128 * F];            // current message / edge-feature weights, transposed [k][f]
     float wb[128 * F];            // current update weights
     float xs[WARPS][128 * TILE];  // per-warp input tile [k][vertex]
     uint16_t nbr_j[WARPS][256];   // per-warp compacted neighbour list of one 256-entry window: vertex ...
-    int8_t nbr_a[WARPS][256];     // ... and weight
+    T nbr_a[WARPS][256];          // ... and weight
     float w_init[64 * 7];
     float w_edge[64 * 8];
     float w_read[128];
@@ -81,23 +115,26 @@ __device__ __forceinline__ void tile_linear(const float* __restrict__ wt, const 
     }
 }
 
-// Visit the non-zeros of adjacency row `arow` (NP int8) with the whole warp; fn(j, a) is warp-uniform.
-template <class Fn>
-__device__ __forceinline__ void for_each_neighbor(const int8_t* __restrict__ arow, int NP, int lane, Fn fn) {
-    const int nchunks = NP / 16;
+// Visit the non-zeros of adjacency row `arow` (NP couplings) with the whole warp; fn(j, a) is warp-uniform.
+template <class T, class Fn>
+__device__ __forceinline__ void for_each_neighbor(const T* __restrict__ arow, int NP, int lane, Fn fn) {
+    using V = typename CouplingVal<T>::type;
+    constexpr int K = sizeof(T) == 1 ? 16 : 4;          // couplings per lane and chunk
+    const int nchunks = NP / K;
     for (int base = 0; base < nchunks; base += 32) {
-        union { uint4 v; int8_t b[16]; } u;
-        u.v = make_uint4(0, 0, 0, 0);
-        if (base + lane < nchunks) u.v = *reinterpret_cast<const uint4*>(arow + (size_t)(base + lane) * 16);
+        V u[K];
 #pragma unroll
-        for (int k = 0; k < 16; ++k) {
-            const int v = u.b[k];
+        for (int k = 0; k < K; ++k) u[k] = 0;
+        if (base + lane < nchunks) load_row(arow + (size_t)(base + lane) * K, u);
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const V v = u[k];
             unsigned m = __ballot_sync(0xffffffffu, v != 0);
             while (m) {
                 const int src = __ffs(m) - 1;
                 m &= m - 1;
-                const int a = __shfl_sync(0xffffffffu, v, src);
-                fn((base + src) * 16 + k, a);
+                const V a = __shfl_sync(0xffffffffu, v, src);
+                fn((base + src) * K + k, a);
             }
         }
     }
@@ -107,33 +144,37 @@ __device__ __forceinline__ void for_each_neighbor(const int8_t* __restrict__ aro
 // a per-warp list (ballot + popc), then handed out eight at a time, so the caller issues eight independent gathers from
 // the L2-resident embeddings before it uses any of them (one dependent L2 round trip per neighbour made the aggregation
 // 90 % of the kernel on ER-500).  fn(j[8], a[8], cnt): entries >= cnt are (0, 0).
-template <class Fn>
-__device__ __forceinline__ void for_each_neighbor8(const int8_t* __restrict__ arow, int NP, int lane, uint16_t* lj, int8_t* la, Fn fn) {
-    const int nchunks = NP / 8;                         // 8-byte chunks: a window of 32 lanes x 8 = 256 entries
+template <class T, class Fn>
+__device__ __forceinline__ void for_each_neighbor8(const T* __restrict__ arow, int NP, int lane, uint16_t* lj, T* la, Fn fn) {
+    using V = typename CouplingVal<T>::type;
+    constexpr int K = sizeof(T) == 1 ? 8 : 4;           // couplings per lane and chunk: a window of 32 x K <= 256 entries
+    const int nchunks = NP / K;
     for (int base = 0; base < nchunks; base += 32) {
-        union { uint2 v; int8_t b[8]; } u;
-        u.v = make_uint2(0, 0);
-        if (base + lane < nchunks) u.v = *reinterpret_cast<const uint2*>(arow + (size_t)(base + lane) * 8);
+        V u[K];
+#pragma unroll
+        for (int k = 0; k < K; ++k) u[k] = 0;
+        if (base + lane < nchunks) load_row(arow + (size_t)(base + lane) * K, u);
         int count = 0;
 #pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            const int v = u.b[k];
+        for (int k = 0; k < K; ++k) {
+            const V v = u[k];
             const unsigned m = __ballot_sync(0xffffffffu, v != 0);
             if (v != 0) {
                 const int pos = count + __popc(m & ((1u << lane) - 1u));
-                lj[pos] = (uint16_t)((base + lane) * 8 + k);
-                la[pos] = (int8_t)v;
+                lj[pos] = (uint16_t)((base + lane) * K + k);
+                la[pos] = (T)v;
             }
             count += __popc(m);
         }
         __syncwarp();
         for (int t = 0; t < count; t += 8) {
-            int j[8], a[8];
+            int j[8];
+            V a[8];
 #pragma unroll
             for (int e = 0; e < 8; ++e) {
                 const bool in = t + e < count;
                 j[e] = in ? (int)lj[t + e] : 0;
-                a[e] = in ? (int)la[t + e] : 0;
+                a[e] = in ? (V)la[t + e] : (V)0;
             }
             fn(j, a, min(8, count - t));
         }
@@ -141,12 +182,15 @@ __device__ __forceinline__ void for_each_neighbor8(const int8_t* __restrict__ ar
     }
 }
 
-__global__ void __launch_bounds__(WARPS * 32, 2)
-mpnn_simt_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const int32_t* __restrict__ graph_idx,
+// (fp32 couplings: sizeof(Smem<float>) = 115 KB, so one CTA per SM fits anyway and the register budget is not halved)
+template <class T>
+__global__ void __launch_bounds__(WARPS * 32, sizeof(T) == 1 ? 2 : 1)
+mpnn_simt_kernel(const GView<T> g, const eco_mpnn_t w, const int B, const int32_t* __restrict__ graph_idx,
                  const float* __restrict__ xn, const float* __restrict__ xg, const float norm_max,
                  float* __restrict__ q_out, int32_t* __restrict__ act_out, float* __restrict__ scratch) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    Smem& S = *reinterpret_cast<Smem*>(smem_raw);
+    using V = typename CouplingVal<T>::type;
+    Smem<T>& S = *reinterpret_cast<Smem<T>*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int N = g.N, NP = g.NP;
     const float* wt = scratch;                                        // transposed weights (header)
@@ -166,7 +210,7 @@ mpnn_simt_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const in
 
     for (int b = blockIdx.x; b < B; b += gridDim.x) {
         const int gi = graph_idx[b];
-        const int8_t* A = g.J + (size_t)gi * NP * NP;
+        const T* A = g.J + (size_t)gi * NP * NP;
         const float* deg = g.deg + (size_t)gi * NP;
         const float* x0 = xn + (size_t)b * 3 * NP;
         const float4 xgl = *reinterpret_cast<const float4*>(xg + (size_t)b * 4);
@@ -202,13 +246,13 @@ mpnn_simt_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const in
                 float ga = 0.f, gb = 0.f;
                 if (i < N) {
                     if (!batched) {
-                        for_each_neighbor(A + (size_t)i * NP, NP, lane, [&](int j, int a) {
+                        for_each_neighbor(A + (size_t)i * NP, NP, lane, [&](int j, V a) {
                             const float af = (float)a;
                             ga += fmaxf(fmaf(af, w0a, P[(size_t)j * F + lane]), 0.f);
                             gb += fmaxf(fmaf(af, w0b, P[(size_t)j * F + lane + 32]), 0.f);
                         });
                     } else
-                    for_each_neighbor8(A + (size_t)i * NP, NP, lane, S.nbr_j[warp], S.nbr_a[warp], [&](const int (&j)[8], const int (&a)[8], int cnt) {
+                    for_each_neighbor8(A + (size_t)i * NP, NP, lane, S.nbr_j[warp], S.nbr_a[warp], [&](const int (&j)[8], const V (&a)[8], int cnt) {
                         float pa[8], pb[8];
 #pragma unroll
                         for (int e = 0; e < 8; ++e) { pa[e] = P[(size_t)j[e] * F + lane]; pb[e] = P[(size_t)j[e] * F + lane + 32]; }
@@ -257,13 +301,13 @@ mpnn_simt_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const in
                     float aa = 0.f, ab = 0.f, ea = 0.f, eb = 0.f;
                     if (i < N) {
                         if (!batched) {
-                            for_each_neighbor(A + (size_t)i * NP, NP, lane, [&](int j, int a) {
+                            for_each_neighbor(A + (size_t)i * NP, NP, lane, [&](int j, V a) {
                                 const float af = (float)a;
                                 aa = fmaf(af, Hc[(size_t)j * F + lane], aa);
                                 ab = fmaf(af, Hc[(size_t)j * F + lane + 32], ab);
                             });
                         } else
-                        for_each_neighbor8(A + (size_t)i * NP, NP, lane, S.nbr_j[warp], S.nbr_a[warp], [&](const int (&j)[8], const int (&a)[8], int cnt) {
+                        for_each_neighbor8(A + (size_t)i * NP, NP, lane, S.nbr_j[warp], S.nbr_a[warp], [&](const int (&j)[8], const V (&a)[8], int cnt) {
                             float ha[8], hb[8];
 #pragma unroll
                             for (int e = 0; e < 8; ++e) { ha[e] = Hc[(size_t)j[e] * F + lane]; hb[e] = Hc[(size_t)j[e] * F + lane + 32]; }
@@ -384,21 +428,36 @@ size_t mpnn_simt_scratch_bytes(int B, int N) {
     return align256(sizeof(float) * ((size_t)WT_FLOATS + (size_t)simt_grid(B) * 4 * NP * F));
 }
 
-int launch_mpnn_simt(const eco_graphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
-                     const float* xg, float norm_max, float* q, int32_t* actions, void* scratch,
-                     cudaStream_t st) {
-    static unsigned long long attr_set = 0;
+namespace {
+template <class T>
+int launch_simt(const GView<T>& g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn, const float* xg,
+                float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st) {
+    static unsigned long long attr_set = 0;     // (one per instantiation)
     if (first_use_on_device(&attr_set))
-        ECO_CUDA(cudaFuncSetAttribute(mpnn_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)sizeof(Smem)));
+        ECO_CUDA(cudaFuncSetAttribute(mpnn_simt_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)sizeof(Smem<T>)));
     transpose_weights_kernel<<<(128 * 64 + 255) / 256, 256, 0, st>>>(*w, (float*)scratch);
     ECO_LAUNCH_CHECK();
     prof_begin(ECO_PROF_MPNN, st);
-    mpnn_simt_kernel<<<simt_grid(B), WARPS * 32, sizeof(Smem), st>>>(*g, *w, B, gidx, xn, xg, norm_max, q,
-                                                                    actions, (float*)scratch);
+    mpnn_simt_kernel<T><<<simt_grid(B), WARPS * 32, sizeof(Smem<T>), st>>>(g, *w, B, gidx, xn, xg, norm_max, q,
+                                                                          actions, (float*)scratch);
     prof_end(ECO_PROF_MPNN, st);
     ECO_LAUNCH_CHECK();
     return ECO_OK;
+}
+}  // namespace
+
+int launch_mpnn_simt(const eco_graphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
+                     const float* xg, float norm_max, float* q, int32_t* actions, void* scratch,
+                     cudaStream_t st) {
+    const GView<int8_t> v{g->J, g->deg, g->gstat, g->dmax, g->N, g->NP};
+    return launch_simt(v, w, B, gidx, xn, xg, norm_max, q, actions, scratch, st);
+}
+
+int launch_mpnn_simt_w(const eco_wgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
+                       const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st) {
+    const GView<float> v{g->Jf, g->deg, g->gstat, g->dmax, g->N, g->NP};
+    return launch_simt(v, w, B, gidx, xn, xg, norm_max, q, actions, scratch, st);
 }
 
 }  // namespace eco

@@ -4,6 +4,7 @@ Host-side mirror of the reference's environment/agent surface for the rollout ho
 
   GraphSet             <- SingleGraphGenerator / SetGraphGenerator payloads (src/envs/utils.py:319-382) +
                           MaximumCutUnbiasedScorer constants (src/envs/score_solver.py:347-375)
+  WeightedGraphSet     <- the same for real-valued couplings (EdgeType.RANDOM): fp64 environment, fp32(J) MPNN
   BatchedSpinSystem    <- B x SpinSystemBase (src/envs/spinsystem.py:50-607): reset / step / observation /
                           best_* trackers, struct-of-arrays on the device
   MPNNWeights          <- MPNN.state_dict() (src/networks/mpnn.py:5-32; SURVEY.md appendix A.3)
@@ -15,7 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import Graphs, Env, Mpnn, check, lib
+from ._lib import Graphs, Env, Mpnn, WGraphs, WEnv, check, lib
 
 STATE_DICT_KEYS = (
     "node_init_embedding_layer.0.weight",
@@ -39,6 +40,9 @@ EPISODE_DTYPE = np.dtype([("step", "<i4"), ("cut", "<i4"), ("best_cut", "<i4"), 
                           ("score", "<f8"), ("nscore", "<f8"), ("best_score", "<f8"), ("best_nscore", "<f8"),
                           ("key", "<u8", (2,)), ("total_reward", "<f8"), ("last_reward", "<f8")])
 assert EPISODE_DTYPE.itemsize == 96
+# BatchedSpinSystem.episodes() of a weighted set: the cut fields are the fp64 cut / best cut of eco_wenv_t
+WEIGHTED_EPISODE_DTYPE = np.dtype([(n, "<f8" if n in ("cut", "best_cut") else EPISODE_DTYPE.fields[n][0])
+                                   for n in EPISODE_DTYPE.names])
 
 
 def _require_cuda(device=None):
@@ -107,7 +111,22 @@ def graphs_to_int8(graphs):
     return np.ascontiguousarray(arr)
 
 
+def is_int8_graph(graphs):
+    """True when every coupling is an integer in [-127, 127] (the int8 path takes it; anything else is a weighted graph)."""
+    arr = np.asarray(graphs)
+    if arr.dtype == np.int8:
+        return True
+    if arr.size == 0:
+        return True
+    if not np.issubdtype(arr.dtype, np.number) or not np.isfinite(arr).all():
+        return False
+    r = np.rint(arr)
+    return bool(np.array_equal(r, arr) and np.abs(r).max(initial=0) <= 127)
+
+
 class GraphSet:
+    weighted = False
+
     def __init__(self, graphs, device=None, validate=True, min_cut=False, _edges=None):
         """min_cut=True: the scorer constants (and every mask the env kernels derive from the graphs) are those of
         OptimisationTarget.MIN_CUT (reference score_solver.py:423-505) instead of CUT.
@@ -199,6 +218,77 @@ class GraphSet:
         return self.gscal[:, 2]
 
 
+class WeightedGraphSet:
+    """G dense symmetric graphs with real-valued couplings (EdgeType.RANDOM: 2*rand-1 weights, or any non-integer matrix a
+    SingleGraphGenerator / SetGraphGenerator / load_graph_set hands over), shared read-only by all episodes.  The environment
+    runs in fp64 on these couplings, as the reference's fp64 `matrix` does; the MPNN reads their fp32 cast, as the
+    reference's drivers do with `.float()` (experiments/utils.py:174).  ECO-DQN configuration (CUT target) only."""
+    weighted = True
+    min_cut = False
+    pm1_only = False
+
+    def __init__(self, graphs, device=None, validate=True):
+        self.device = _require_cuda(device)
+        arr = np.asarray(graphs, dtype=np.float64)
+        if arr.ndim == 2:
+            arr = arr[None]
+        if arr.ndim != 3 or arr.shape[1] != arr.shape[2]:
+            raise ValueError("graphs must be [G, N, N] (all graphs of one set share N), got shape %s" % (arr.shape,))
+        self.G, self.N = int(arr.shape[0]), int(arr.shape[1])
+        if self.N > _lib.MAX_SPINS:
+            raise ValueError("N=%d exceeds ECO_MAX_SPINS=%d" % (self.N, _lib.MAX_SPINS))
+        if self.G < 1 or self.N < 1:
+            raise ValueError("empty graph set")
+        L = lib()
+        with torch.cuda.device(self.device):
+            self._ws = torch.zeros(L.eco_wgraphs_workspace_bytes(self.G, self.N), dtype=torch.uint8, device=self.device)
+            self.c = WGraphs()
+            check(L.eco_wgraphs_bind(C.byref(self.c), _ptr(self._ws), self.G, self.N))
+            Jd = torch.from_numpy(np.ascontiguousarray(arr)).to(self.device)
+            check(L.eco_wgraphs_load_dev(C.byref(self.c), _ptr(Jd), _stream()))
+            self.NP = int(self.c.NP)
+            G, NP = self.G, self.NP
+            self.J = _view(self._ws, self.c.J, G * NP * NP, torch.float64, (G, NP, NP))
+            self.Jf = _view(self._ws, self.c.Jf, G * NP * NP, torch.float32, (G, NP, NP))
+            self.gscal = _view(self._ws, self.c.gscal, G * 4, torch.float64, (G, 4))
+            self.deg = _view(self._ws, self.c.deg, G * NP, torch.float32, (G, NP))
+            self.gstat = _view(self._ws, self.c.gstat, G * 4, torch.int32, (G, 4))
+            stat = self.gstat.cpu().numpy()
+        self.max_degree = int(stat[:, 0].max())
+        if validate:
+            first = lambda bit: int(np.nonzero(stat[:, 3] & bit)[0][0])
+            if (stat[:, 3] & _lib.WGRAPH_NONFINITE).any():
+                raise ValueError("graph %d has a non-finite coupling" % first(_lib.WGRAPH_NONFINITE))
+            if (stat[:, 3] & _lib.WGRAPH_ASYMMETRIC).any():
+                raise ValueError("graph %d is not symmetric with a zero diagonal" % first(_lib.WGRAPH_ASYMMETRIC))
+            if (stat[:, 3] & _lib.WGRAPH_NO_DEGREE).any():
+                # the reference recurses forever on such a graph (spinsystem.py:209-211)
+                raise ValueError("graph %d has no non-zero weighted degree" % first(_lib.WGRAPH_NO_DEGREE))
+
+    @property
+    def mlr(self):
+        return self.gscal[:, 0]
+
+    @property
+    def qn(self):
+        return self.gscal[:, 1]
+
+    @property
+    def lb(self):
+        return self.gscal[:, 2]
+
+
+def graph_set(graphs, device=None, validate=True, min_cut=False):
+    """GraphSet when every coupling is an integer in [-127, 127], WeightedGraphSet otherwise (what the drop-in surface
+    routes through: integer graphs keep the int8 path and its results bit for bit)."""
+    if is_int8_graph(graphs):
+        return GraphSet(graphs, device=device, validate=validate, min_cut=min_cut)
+    if min_cut:
+        raise NotImplementedError("OptimisationTarget.MIN_CUT with real-valued couplings is not supported "
+                                  "(weighted graphs run the CUT target only)")
+    return WeightedGraphSet(graphs, device=device, validate=validate)
+
+
 class MPNNWeights:
     """fp32 device copies of the 12 reference tensors + the C struct pointing at them."""
 
@@ -267,34 +357,52 @@ class BatchedSpinSystem:
             raise ValueError("n_envs must be >= 1")
         if not (1 <= self.T <= 65535):
             raise ValueError("max_steps must be in [1, 65535]")
+        # real-valued couplings: fp64 fields (eco_wenv_t), ECO-DQN configuration only
+        self.weighted = bool(getattr(graphset, "weighted", False))
+        if self.weighted and (not reversible_spins or dense_reward):
+            raise NotImplementedError("irreversible spins / dense reward (S2V-DQN) with real-valued couplings are not "
+                                      "supported: weighted graphs run the ECO-DQN configuration only")
         self.basin_reward = basin_reward
         self.mpnn_impl = mpnn_impl
         L = lib()
+        basin = float(basin_reward) if basin_reward is not None else -1.0
         with torch.cuda.device(self.device):
-            nbytes = L.eco_env_workspace_bytes(self.B, self.N, self.T)
-            self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
-            self.c = Env()
-            check(L.eco_env_bind(C.byref(self.c), _ptr(self._ws), self.B, self.N, self.T,
-                                 float(basin_reward) if basin_reward is not None else -1.0))
-            self.NP, self.NW = int(self.c.NP), int(self.c.NW)
+            if self.weighted:
+                nbytes = L.eco_wenv_workspace_bytes(self.B, self.N, self.T)
+                self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
+                self.c = WEnv()
+                check(L.eco_wenv_bind(C.byref(self.c), _ptr(self._ws), self.B, self.N, self.T, basin))
+                self._base = self.c.base        # (shares the memory of self.c)
+            else:
+                nbytes = L.eco_env_workspace_bytes(self.B, self.N, self.T)
+                self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
+                self.c = Env()
+                check(L.eco_env_bind(C.byref(self.c), _ptr(self._ws), self.B, self.N, self.T, basin))
+                self._base = self.c
+            base = self._base
+            self.NP, self.NW = int(base.NP), int(base.NW)
             self.reversible_spins, self.dense_reward = bool(reversible_spins), bool(dense_reward)
-            self.c.reserved = (0 if reversible_spins else _lib.ENV_IRREVERSIBLE) | (_lib.ENV_DENSE_REWARD if dense_reward else 0)
+            base.reserved = (0 if reversible_spins else _lib.ENV_IRREVERSIBLE) | (_lib.ENV_DENSE_REWARD if dense_reward else 0)
             zob = np.ascontiguousarray(zobrist_keys(self.NP))
             tsf = time_since_flip_table(self.T).astype(np.float32)
             imm = immanency_table(self.T).astype(np.float32)
-            check(L.eco_env_set_tables(C.byref(self.c), zob.ctypes.data_as(C.c_void_p), tsf.ctypes.data_as(C.c_void_p),
+            check(L.eco_env_set_tables(C.byref(base), zob.ctypes.data_as(C.c_void_p), tsf.ctypes.data_as(C.c_void_p),
                                        imm.ctypes.data_as(C.c_void_p), _stream()))
             torch.cuda.current_stream().synchronize()   # host tables are temporaries
             B, NP = self.B, self.NP
             ws = self._ws
-            self.spins = _view(ws, self.c.spins, B * NP, torch.int8, (B, NP))
-            self.hfield = _view(ws, self.c.hfield, B * NP, torch.int16, (B, NP))
-            self.last_flip = _view(ws, self.c.last_flip, B * NP, torch.int16, (B, NP))
-            self.diff_bits = _view(ws, self.c.diff_bits, B * self.NW, torch.int32, (B, self.NW))
-            self.graph_idx = _view(ws, self.c.graph_idx, B, torch.int32, (B,))
-            self._ep = _view(ws, self.c.ep, B * 96, torch.uint8, (B, 96))
-            self.xn = _view(ws, self.c.xn, B * 3 * NP, torch.float32, (B, 3, NP))
-            self.xg = _view(ws, self.c.xg, B * 4, torch.float32, (B, 4))
+            self.spins = _view(ws, base.spins, B * NP, torch.int8, (B, NP))
+            if self.weighted:
+                self.hfield = _view(ws, self.c.h, B * NP, torch.float64, (B, NP))
+                self.cuts = _view(ws, self.c.cut, B * 2, torch.float64, (B, 2))     # current cut, best cut
+            else:
+                self.hfield = _view(ws, base.hfield, B * NP, torch.int16, (B, NP))
+            self.last_flip = _view(ws, base.last_flip, B * NP, torch.int16, (B, NP))
+            self.diff_bits = _view(ws, base.diff_bits, B * self.NW, torch.int32, (B, self.NW))
+            self.graph_idx = _view(ws, base.graph_idx, B, torch.int32, (B,))
+            self._ep = _view(ws, base.ep, B * 96, torch.uint8, (B, 96))
+            self.xn = _view(ws, base.xn, B * 3 * NP, torch.float32, (B, 3, NP))
+            self.xg = _view(ws, base.xg, B * 4, torch.float32, (B, 4))
             self._actions = torch.zeros(B, dtype=torch.int32, device=self.device)
             self._reward = torch.zeros(B, dtype=torch.float64, device=self.device)
             self._done = torch.zeros(B, dtype=torch.uint8, device=self.device)
@@ -335,7 +443,8 @@ class BatchedSpinSystem:
             if int(gi.min()) < 0 or int(gi.max()) >= self.gs.G:
                 raise ValueError("graph_idx out of range")
         with torch.cuda.device(self.device):
-            check(lib().eco_env_reset(C.byref(self.gs.c), C.byref(self.c), _ptr(gi), _ptr(sp), _stream()))
+            reset = lib().eco_wenv_reset if self.weighted else lib().eco_env_reset
+            check(reset(C.byref(self.gs.c), C.byref(self.c), _ptr(gi), _ptr(sp), _stream()))
         self.current_step = 0
         self._is_reset = True
         return self
@@ -354,8 +463,9 @@ class BatchedSpinSystem:
         if a.shape != (self.B,):
             raise ValueError("actions must be [B]")
         ha, hr, hs = hist if hist is not None else (None, None, None)
+        step = lib().eco_wenv_step if self.weighted else lib().eco_env_step
         with torch.cuda.device(self.device):
-            check(lib().eco_env_step(C.byref(self.gs.c), C.byref(self.c), _lib.POLICY_ACTIONS, _ptr(a),
+            check(step(C.byref(self.gs.c), C.byref(self.c), _lib.POLICY_ACTIONS, _ptr(a),
                                      _ptr(self._reward), _ptr(self._done), _ptr(ha), _ptr(hr), _ptr(hs), _stream()))
         self.current_step += 1
         return self._reward, self._done
@@ -364,8 +474,9 @@ class BatchedSpinSystem:
         """One step of the Greedy solver (src/agents/solver.py:105-131) for every episode still running."""
         self._check_steppable()
         ha, hr, hs = hist if hist is not None else (None, None, None)
+        step = lib().eco_wenv_step if self.weighted else lib().eco_env_step
         with torch.cuda.device(self.device):
-            check(lib().eco_env_step(C.byref(self.gs.c), C.byref(self.c), _lib.POLICY_GREEDY, None,
+            check(step(C.byref(self.gs.c), C.byref(self.c), _lib.POLICY_GREEDY, None,
                                      _ptr(self._reward), _ptr(self._done), _ptr(ha), _ptr(hr), _ptr(hs), _stream()))
         self.current_step += 1
         return self._reward, self._done
@@ -382,8 +493,9 @@ class BatchedSpinSystem:
         q = torch.zeros(self.B, self.NP, dtype=torch.float32, device=self.device)
         acts = self._actions if want_actions else None
         nm = float(norm_max) if norm_max is not None else 0.0
+        forward = lib().eco_wmpnn_forward if self.weighted else lib().eco_mpnn_forward
         with torch.cuda.device(self.device):
-            check(lib().eco_mpnn_forward(C.byref(self.gs.c), C.byref(weights.c), self.B, _ptr(self.graph_idx),
+            check(forward(C.byref(self.gs.c), C.byref(weights.c), self.B, _ptr(self.graph_idx),
                                          _ptr(self.xn), _ptr(self.xg), nm, _ptr(q), _ptr(acts),
                                          _ptr(self._scratch_for(self.B)), self.mpnn_impl if impl is None else impl,
                                          _stream()))
@@ -411,8 +523,9 @@ class BatchedSpinSystem:
         if pol == _lib.POLICY_NETWORK and weights is None:
             raise ValueError("network policy needs weights")
         nm = float(norm_max) if norm_max is not None else -1.0
+        rollout = lib().eco_wrollout if self.weighted else lib().eco_rollout
         with torch.cuda.device(self.device):
-            check(lib().eco_rollout(C.byref(self.gs.c), C.byref(self.c),
+            check(rollout(C.byref(self.gs.c), C.byref(self.c),
                                     C.byref(weights.c) if weights is not None else None, n_steps, pol, nm,
                                     _ptr(self._actions),
                                     _ptr(self._scratch_for(self.B)) if pol == _lib.POLICY_NETWORK else None,
@@ -427,20 +540,30 @@ class BatchedSpinSystem:
         The adjacency rows 7.. are the (static) graph and are never materialised per step."""
         obs = torch.empty(self.B, 7, self.N, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            check(lib().eco_env_observation(C.byref(self.c), _ptr(obs), _stream()))
+            check(lib().eco_env_observation(C.byref(self._base), _ptr(obs), _stream()))
         return obs
 
     def episodes(self):
-        """Per-episode scalar blocks as a numpy structured array (synchronises)."""
-        return self._ep.cpu().numpy().view(EPISODE_DTYPE).reshape(self.B)
+        """Per-episode scalar blocks as a numpy structured array (synchronises).  Weighted sets: `cut` / `best_cut` are
+        the fp64 values."""
+        ep = self._ep.cpu().numpy().view(EPISODE_DTYPE).reshape(self.B)
+        if not self.weighted:
+            return ep
+        out = np.zeros(self.B, dtype=WEIGHTED_EPISODE_DTYPE)
+        for n in EPISODE_DTYPE.names:
+            out[n] = ep[n]
+        cuts = self.cuts.cpu().numpy()
+        out["cut"], out["best_cut"] = cuts[:, 0], cuts[:, 1]
+        return out
 
     def results(self):
-        """(best_cut int32 [B], best_spins int8 [B, N], steps int32 [B]) device tensors."""
-        bc = torch.empty(self.B, dtype=torch.int32, device=self.device)
+        """(best_cut int32 [B] -- fp64 for a weighted set --, best_spins int8 [B, N], steps int32 [B]) device tensors."""
+        bc = torch.empty(self.B, dtype=torch.float64 if self.weighted else torch.int32, device=self.device)
         bs = torch.empty(self.B, self.N, dtype=torch.int8, device=self.device)
         st = torch.empty(self.B, dtype=torch.int32, device=self.device)
+        results = lib().eco_wenv_results if self.weighted else lib().eco_env_results
         with torch.cuda.device(self.device):
-            check(lib().eco_env_results(C.byref(self.c), _ptr(bc), _ptr(bs), _ptr(st), _stream()))
+            check(results(C.byref(self.c), _ptr(bc), _ptr(bs), _ptr(st), _stream()))
         return bc, bs, st
 
 
@@ -465,6 +588,9 @@ class HostSession:
             if x is None:
                 return C.c_void_p(0)
             return C.c_void_p(x.data_ptr()) if torch.is_tensor(x) else x.ctypes.data_as(C.c_void_p)
+        if J_host is not None and not is_int8_graph(J_host.cpu().numpy() if torch.is_tensor(J_host) else J_host):
+            raise NotImplementedError("HostSession takes int8 couplings only; real-valued graphs run through "
+                                      "WeightedGraphSet + BatchedSpinSystem")
         pol = {"network": _lib.POLICY_NETWORK, "greedy": _lib.POLICY_GREEDY}[policy]
         check(lib().eco_session_rollout(self._h, hp(J_host), hp(graph_idx_host), hp(init_spins_host), pol,
                                         float(norm_max) if norm_max is not None else -1.0, hp(best_cut_out),

@@ -190,8 +190,9 @@ class SpinSystemBase:
     def _bind_graph(self, matrix):
         key = (id(matrix), matrix.shape)
         if self._graphset is None or key != self._graph_key:
-            self._graphset = engine.GraphSet(np.asarray(matrix)[None], device=self._device,
-                                             min_cut=self.optimisation_target == OptimisationTarget.MIN_CUT)
+            # integer couplings in [-127, 127]: the int8 path; anything else (EdgeType.RANDOM): the fp64 weighted path
+            self._graphset = engine.graph_set(np.asarray(matrix)[None], device=self._device,
+                                              min_cut=self.optimisation_target == OptimisationTarget.MIN_CUT)
             self._graph_key = key
             self._env = self._new_env()
             sc = self._graphset.gscal.cpu().numpy()[0]

@@ -80,8 +80,9 @@ def test_network(network, env_args, graphs_test, device=None, step_factor=1, bat
     for n, idxs in groups.items():
         n_steps = int(n * step_factor)
         args = _check_env_args(env_args, n_steps)
-        gs = engine.GraphSet(np.stack([graphs_test[j] for j in idxs]), device=dev,
-                             min_cut=args["optimisation_target"] == OptimisationTarget.MIN_CUT)
+        # integer couplings in [-127, 127]: the int8 path; anything else (EdgeType.RANDOM): the fp64 weighted path
+        gs = engine.graph_set(np.stack([graphs_test[j] for j in idxs]), device=dev,
+                              min_cut=args["optimisation_target"] == OptimisationTarget.MIN_CUT)
         G = len(idxs)
         B = G * n_attempts
         gidx = np.repeat(np.arange(G, dtype=np.int32), n_attempts)
@@ -214,13 +215,14 @@ def load_graph_set(graph_save_loc):
 def load_graph_set_device(graph_save_loc, device=None, min_cut=False):
     """The same pickle straight into an engine.GraphSet (all graphs of the file must share N, as the reference's batched
     tester assumes per graph anyway).  A file of scipy sparse matrices (the csr pickles) goes through the sparse ingest --
-    only the stored entries cross PCIe, the dense int8 couplings are built on the device; anything else is uploaded as int8."""
+    only the stored entries cross PCIe, the dense int8 couplings are built on the device; anything else is uploaded as int8,
+    or, when a coupling is not an integer in [-127, 127], as an fp64 engine.WeightedGraphSet."""
     with open(graph_save_loc, 'rb') as f:
         raw = pickle.load(f)
     if len(raw) and all(sp.sparse.issparse(g) for g in raw):
         return engine.GraphSet.from_edges(raw[0].shape[0], raw, device=device, min_cut=min_cut)
     graphs = [to_dense_adjacency(g) for g in raw]
-    return engine.GraphSet(engine.graphs_to_int8(np.stack(graphs)), device=device, min_cut=min_cut)
+    return engine.graph_set(np.stack(graphs), device=device, min_cut=min_cut)
 
 
 def load_mc_instances_device(graph_dir, graph_names, device=None, min_cut=False):

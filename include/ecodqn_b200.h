@@ -15,8 +15,9 @@
  *     last failure on the calling thread.  Shape / configuration violations are rejected before any launch.
  *   - All work is enqueued asynchronously on `stream`; no entry point synchronises unless it says so.
  *   - Vertices are padded to NP = 16*ceil(N/16) per row; padded entries are zero and never selected.
- *   - Integer-weight graphs only (int8 couplings; the reference's EdgeType.UNIFORM / DISCRETE).  There is no
- *     CPU fallback anywhere in this library.
+ *   - Integer-weight graphs (int8 couplings; the reference's EdgeType.UNIFORM / DISCRETE) through eco_graphs_t, and
+ *     real-valued graphs (fp64 couplings; EdgeType.RANDOM) through the eco_wgraphs_t / eco_wenv_t entry points at the
+ *     end of this header.  There is no CPU fallback anywhere in this library.
  */
 #ifndef ECODQN_B200_H
 #define ECODQN_B200_H
@@ -326,6 +327,68 @@ int64_t eco_launch_count(int reset);
 #define ECO_PROF_ROLLOUT 2
 int eco_profile_enable(int on);
 int eco_profile_read(int kind, double* total_ms, int64_t* launches);
+
+/* ---------------------------------------------------------------------------------------------------------
+ * Real-valued couplings (EdgeType.RANDOM: 2*rand-1 weights, reference src/envs/utils.py; any non-integer matrix of
+ * SingleGraphGenerator / SetGraphGenerator / load_graph_set).  ECO-DQN rollout configuration only (CUT target, BLS
+ * reward, reversible spins) plus the Greedy baseline.  Precision follows the reference:
+ *   - the environment is fp64 (couplings, local fields, gains, score, normalised score, cut, rewards), as
+ *     spinsystem.py computes with its fp64 `matrix`;
+ *   - the MPNN reads fp32(J), because the reference's drivers cast the observation with .float()
+ *     (experiments/utils.py:174): degree = #{j : fp32(J_ij) != 0}, edge stage and aggregation on fp32 couplings.
+ * The tensor-core MPNN kernels stay {-1,0,1}-only: ECO_MPNN_TCGEN05 on a weighted set is ECO_ERR_UNSUPPORTED.
+ * --------------------------------------------------------------------------------------------------------- */
+#define ECO_WGRAPH_NO_DEGREE   2   /* gstat flag: every weighted degree is zero (the reference recurses forever)       */
+#define ECO_WGRAPH_ASYMMETRIC  4   /* gstat flag: not symmetric, or a non-zero diagonal entry                          */
+#define ECO_WGRAPH_NONFINITE   8   /* gstat flag: an entry is inf or nan                                               */
+
+typedef struct {
+    int32_t  G, N, NP, reserved;   /* reserved: 0 (OptimisationTarget.CUT only)                                        */
+    double*  J;          /* [G, NP, NP]  fp64 couplings, zero padded                                               */
+    float*   Jf;         /* [G, NP, NP]  fp32(J): what the MPNN reads                                              */
+    double*  gscal;      /* [G, 4]       mlr (max non-zero weighted degree), qn, lb, sum_ij J_ij (score_solver.py:353-375) */
+    float*   deg;        /* [G, NP]      max(1, #{j : fp32(J_ij) != 0})  (mpnn.py:34-38 on the fp32 observation)    */
+    int32_t* gstat;      /* [G, 4]       max degree, nnz, 0, ECO_WGRAPH_* flags                                    */
+    float*   dmax;       /* [1]          max degree over the whole set                                             */
+} eco_wgraphs_t;
+
+size_t eco_wgraphs_workspace_bytes(int32_t G, int32_t N);
+int    eco_wgraphs_bind(eco_wgraphs_t* g, void* workspace_dev, int32_t G, int32_t N);
+/* J_dev: dense [G, N, N] fp64 on the device.  Pads, writes the fp32 copy, the degrees, the flags and the scorer constants
+ * in fp64 (replaces MaximumCutUnbiasedScorer.set_graph, score_solver.py:353-375, and mpnn.py:34-38). */
+int    eco_wgraphs_load_dev(eco_wgraphs_t* g, const double* J_dev, void* stream);
+
+/* Batched environment on a weighted set: the integer state `base` plus the fp64 arrays it cannot hold.  base.hfield and
+ * the cut fields of base.ep are unused; every other array of `base` keeps its meaning, so eco_env_set_tables,
+ * eco_env_observation, eco_env_best_spins and eco_env_masked_argmax take &base. */
+typedef struct {
+    eco_env_t base;
+    double*   h;         /* [B, NP]  local fields h = J s in fp64                                                  */
+    double*   cut;       /* [B, 2]   current cut, best cut (best_solution)                                         */
+} eco_wenv_t;
+
+size_t eco_wenv_workspace_bytes(int32_t B, int32_t N, int32_t T);
+int    eco_wenv_bind(eco_wenv_t* env, void* workspace_dev, int32_t B, int32_t N, int32_t T, double basin_reward);
+/* reset(spins): reference spinsystem.py:183-259 / 283-330, arguments as eco_env_reset */
+int    eco_wenv_reset(const eco_wgraphs_t* g, eco_wenv_t* env, const int32_t* graph_idx_dev, const int8_t* init_spins_dev,
+                      void* stream);
+/* step: reference spinsystem.py:355-559 (ECO_POLICY_ACTIONS) or solver.py:105-131 (ECO_POLICY_GREEDY, key s_i h_i in
+ * fp64, stop when the best gain is < 0); arguments and history arrays as eco_env_step */
+int    eco_wenv_step(const eco_wgraphs_t* g, eco_wenv_t* env, int32_t policy, const int32_t* actions_dev, double* reward_dev,
+                     uint8_t* done_dev, int32_t* hist_actions_dev, double* hist_rewards_dev, double* hist_scores_dev,
+                     void* stream);
+/* MPNN.forward (mpnn.py:40-159) on fp32(J) + argmax; arguments and norm_max modes as eco_mpnn_forward.  impl: AUTO or SIMT. */
+int    eco_wmpnn_forward(const eco_wgraphs_t* g, const eco_mpnn_t* w, int32_t B, const int32_t* graph_idx_dev,
+                         const float* xn_dev, const float* xg_dev, float norm_max, float* q_dev, int32_t* actions_dev,
+                         void* scratch_dev, int32_t impl, void* stream);
+/* rollout: experiments/utils.py:169-207 (ECO_POLICY_NETWORK) or :218-227 (ECO_POLICY_GREEDY); arguments as eco_rollout,
+ * scratch sized by eco_mpnn_scratch_bytes(B, N, ECO_MPNN_SIMT) */
+int    eco_wrollout(const eco_wgraphs_t* g, eco_wenv_t* env, const eco_mpnn_t* w, int32_t n_steps, int32_t policy,
+                    float norm_max, int32_t* actions_scratch_dev, void* mpnn_scratch_dev, int32_t impl,
+                    int32_t* hist_actions_dev, double* hist_rewards_dev, double* hist_scores_dev, void* stream);
+/* best cut (fp64), best spins [B, N] int8, step count.  Any may be NULL. */
+int    eco_wenv_results(const eco_wenv_t* env, double* best_cut_dev, int8_t* best_spins_dev, int32_t* steps_dev,
+                        void* stream);
 
 #ifdef __cplusplus
 }
