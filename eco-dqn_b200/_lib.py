@@ -12,6 +12,7 @@ MPNN_AUTO, MPNN_SIMT, MPNN_TCGEN05 = 0, 1, 2
 MPNN_N_PARAMS = 58425
 LOSS_MSE, LOSS_HUBER = 0, 1
 ENV_IRREVERSIBLE, ENV_DENSE_REWARD = 1, 2      # eco_env_t.reserved mode bits (include/ecodqn_b200.h)
+GRAPHS_PM1 = 1                                  # eco_graphs_t.reserved: every coupling in {-1,0,1}
 GRAPHS_MIN_CUT = 2                              # eco_graphs_t.reserved: OptimisationTarget.MIN_CUT
 MAX_SPINS = 2048
 

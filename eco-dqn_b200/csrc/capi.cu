@@ -413,7 +413,7 @@ int eco_mpnn_grad_ev(const eco_graphs_t* g, const eco_mpnn_t* w, int32_t B, cons
     ECO_CHECK_ARG(B >= 1 && B <= 65535, ECO_ERR_INVALID, "eco_mpnn_grad: B must be in 1..65535 (minibatch), got %d", B);
     ECO_CHECK_ARG(loss_kind == ECO_LOSS_MSE || loss_kind == ECO_LOSS_HUBER, ECO_ERR_INVALID, "eco_mpnn_grad: unknown loss %d",
                   loss_kind);
-    ECO_CHECK_ARG(g->reserved & 1, ECO_ERR_UNSUPPORTED, "eco_mpnn_grad: needs couplings in {-1,0,1}");
+    ECO_CHECK_ARG(g->reserved & ECO_GRAPHS_PM1, ECO_ERR_UNSUPPORTED, "eco_mpnn_grad: needs couplings in {-1,0,1}");
     ECO_CHECK_ARG((((uintptr_t)scratch | (uintptr_t)grad) & 15) == 0, ECO_ERR_INVALID, "eco_mpnn_grad: scratch and grad must be 16-byte aligned");
     int rc = check_weights(w, "eco_mpnn_grad");
     if (rc) return rc;
@@ -729,7 +729,7 @@ int eco_session_rollout(eco_session_t* s, const int8_t* J_host, const int32_t* g
         for (int i = 0; i < s->G; ++i) flags |= stat[(size_t)i * 4 + 3];
         ECO_CHECK_ARG(!(flags & 6), ECO_ERR_INVALID,
                       "eco_session_rollout: a graph is not symmetric with zero diagonal, or has no non-zero degree");
-        s->graphs.reserved = (flags & 1) ? 0 : 1;
+        s->graphs.reserved = (flags & 1) ? 0 : ECO_GRAPHS_PM1;
         if (s->impl != ECO_MPNN_SIMT && !s->w.packed && eco_mpnn_packed_bytes() > 0) {
             rc = eco_mpnn_pack(&s->w, s->packed_buf, stream);
             if (rc) return rc;

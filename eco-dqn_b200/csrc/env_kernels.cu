@@ -278,8 +278,8 @@ env_step_sw_kernel(const eco_graphs_t g, const eco_env_t env, const int policy, 
 // stream filled with 16-byte asynchronous copies (cp.async, one commit group per episode).  While episode e is processed
 // from shared memory, the copies of episode e+2 -- spins, local fields, last-flip steps, the scalar block and row `a` of
 // its adjacency -- are already in flight, so no global-load latency sits on the per-episode path.
-// Same arithmetic as env_step_kernel (bit-exact); caller-supplied actions only (the greedy policy needs the fields to
-// pick the row).
+// Same arithmetic as env_step_kernel (bit-exact; the fp64 bookkeeping is bls_step_scalars); caller-supplied actions only
+// (the greedy policy needs the fields to pick the row).
 namespace tma {
 __device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 }  // namespace tma
@@ -310,7 +310,7 @@ env_step_ring_kernel(const eco_graphs_t g, const eco_env_t env, const int32_t* _
     const int N = env.N, NP = env.NP, NCH = NP >> 3;
     const int stage_bytes = 6 * NP + (int)sizeof(eco_episode_t);
     unsigned char* my_ring = ring_raw + (size_t)stream * STAGES * stage_bytes;
-    const bool use_tab = (g.reserved & 1) != 0;
+    const bool use_tab = (g.reserved & ECO_GRAPHS_PM1) != 0;
     // the two tables every episode indexes with data-dependent addresses live in shared memory (L2 latency otherwise
     // sits between the loads and the first feature store / the visited-set probe)
     __shared__ __align__(16) uint64_t s_zob[2 * 256];
@@ -405,11 +405,11 @@ env_step_ring_kernel(const eco_graphs_t g, const eco_env_t env, const int32_t* _
         const float* gtab = g.gain_tab + (size_t)gi * tab_stride(NP) + NP;
 
         // lanes 0 / 16: scalar state, dependent lookups requested now, used after the vertex loop
-        double sc0 = 0, sc1 = 0, sc2 = 0, sc3 = 0, total_reward = 0, delta_n = 0, qn = 1.0;
+        double sc[4] = {0, 0, 0, 0}, total_reward = 0, delta_n = 0, qn = 1.0;
         ulonglong2 key = make_ulonglong2(0, 0), zob = make_ulonglong2(0, 0);
         uint32_t old_word = 0;
         if (l16 == 0 && valid) {
-            sc0 = S_ep->score; sc1 = S_ep->nscore; sc2 = S_ep->best_score; sc3 = S_ep->best_nscore;
+            sc[0] = S_ep->score; sc[1] = S_ep->nscore; sc[2] = S_ep->best_score; sc[3] = S_ep->best_nscore;
             key = make_ulonglong2(S_ep->key[0], S_ep->key[1]);
             total_reward = S_ep->total_reward;
             zob = *reinterpret_cast<const ulonglong2*>(s_zob + 2 * a);
@@ -425,7 +425,10 @@ env_step_ring_kernel(const eco_graphs_t g, const eco_env_t env, const int32_t* _
         if (l16 == 0 && active && env.use_basin) tv = *reinterpret_cast<const ulonglong2*>(tab + 2 * slot);
 
         int nimp = 0;
-        const SmallDiv gd = small_div_setup(mlr, FAST);   // (not ok: a graph without edges, mlr = 0 -- the general loop divides in fp64)
+        // FAST: gd.ok always holds (couplings in {-1,0,1} give |mlr| <= 255; graph_prepare_kernel sets mlr = 1 when no row sum
+        // is non-zero), so FAST never reaches the general loop below.  It stays compiled in on purpose: without it ptxas
+        // rebuilds the shared-memory window base in every pass of the FAST loop, 3 us (1.3 %) per launch at B = 262 144.
+        const SmallDiv gd = small_div_setup(mlr, FAST);
         // Vertex loop: a lane takes FOUR consecutive vertices per pass (quad qd = l16 + TPE * pass), so the 16 lanes of a stream
         // write 256 contiguous bytes of every feature row with one store instruction -- whole 32-byte sectors.  (With eight
         // vertices per lane the two float4 stores of a row each filled HALF of every sector they touched: twice the write
@@ -513,36 +516,19 @@ env_step_ring_kernel(const eco_graphs_t g, const eco_env_t env, const int32_t* _
         eco_episode_t* ep = env.ep + (valid ? b : 0);
         if (l16 == 0 && active) {
             if (!use_tab) delta_n = __ddiv_rn((double)delta, qn);           // :394
-            const double score = __dadd_rn(sc0, (double)delta);             // :399
-            const double nscore = __dadd_rn(sc1, delta_n);                  // :400
-            const double best_score = sc2, best_nscore = sc3;
             const int cut = e0.y + delta;
-            double rew = 0.0;
-            if (score > best_score) rew = __dsub_rn(nscore, best_nscore);   // :418-424
-            int n_visited = e1.z;
-            if (env.use_basin) {                                            // :443-457
-                const uint64_t w0 = k0 ^ VISITED_SALT0, w1 = k1 ^ VISITED_SALT1;
-                bool is_new = false;
-                for (int probe = 0; probe < env.HCAP; ++probe) {
-                    if (tv.x == 0 && tv.y == 0) {
-                        *reinterpret_cast<ulonglong2*>(tab + 2 * slot) = make_ulonglong2(w0, w1);
-                        is_new = true; ++n_visited;
-                        break;
-                    }
-                    if (tv.x == w0 && tv.y == w1) break;
-                    slot = (slot + 1) & (env.HCAP - 1);
-                    tv = *reinterpret_cast<const ulonglong2*>(tab + 2 * slot);
-                }
-                if (nimp == 0 && is_new) rew = __dadd_rn(rew, env.basin_reward);
-            }
+            const StepScalars r = bls_step_scalars(env, sc, (double)delta, delta_n, nimp, e1.z, tab, slot, tv, k0, k1);
+            const double score = r.score, nscore = r.nscore, rew = r.rew;
             int dist = e0.w + (((old_word >> (a & 31)) & 1u) ? -1 : 1);
             int best_cut = e0.z;
-            double nbs = best_score, nbn = best_nscore;
-            if (score > best_score) { nbs = score; nbn = nscore; best_cut = cut; dist = 0; new_best = 1; }   // :459-463
+            double nbs = sc[2], nbn = sc[3];
+            // (a rarely taken branch instead of r.best_score / r.best_nscore: compiled as selects, this tail made the general
+            // instantiation 0.8 % slower on a B200)
+            if (__builtin_expect(r.new_best, 0)) { nbs = score; nbn = nscore; best_cut = cut; dist = 0; new_best = 1; }
             const int done = step_new == env.T;                             // :541-544
             int4* epw = reinterpret_cast<int4*>(ep);
             epw[0] = make_int4(step_new, cut, best_cut, dist);
-            epw[1] = make_int4(nimp, flags | (done ? FLAG_DONE : 0), n_visited, 0);
+            epw[1] = make_int4(nimp, flags | (done ? FLAG_DONE : 0), r.n_visited, 0);
             *reinterpret_cast<double2*>(&ep->score) = make_double2(score, nscore);
             *reinterpret_cast<double2*>(&ep->best_score) = make_double2(nbs, nbn);
             *reinterpret_cast<ulonglong2*>(&ep->key[0]) = make_ulonglong2(k0, k1);
@@ -726,7 +712,7 @@ int launch_env_step(const eco_graphs_t* g, eco_env_t* env, int policy, const int
                 long long blocks = (B_ + NSTREAMS - 1) / NSTREAMS;
                 if (blocks > (long long)n_sm * 4) blocks = (long long)n_sm * 4;
                 // the stripped vertex loop: +-1 couplings (|gain| <= 255, |mlr| <= 255: small_div is exact), table in shared memory
-                const bool fast = (g->reserved & 1) && env->T + 1 <= TMA_TSF_MAX;
+                const bool fast = (g->reserved & ECO_GRAPHS_PM1) && env->T + 1 <= TMA_TSF_MAX;
                 if (fast) env_step_ring_kernel<TPE, STAGES, true><<<(unsigned)blocks, TMA_WARPS * 32, ring_bytes, st>>>(*g, *env, actions, reward, done, ha, hr, hs);
                 else env_step_ring_kernel<TPE, STAGES, false><<<(unsigned)blocks, TMA_WARPS * 32, ring_bytes, st>>>(*g, *env, actions, reward, done, ha, hr, hs);
             } else ECO_SW(32);

@@ -64,7 +64,7 @@ __device__ __forceinline__ int zx16(uint32_t w, int hh) { return (int)prmt(w, 0,
 // score / normalised score (spinsystem.py:399-400), BLS reward (:418-424), basin reward through the visited set (:443-457),
 // best tracking (:459-463).  delta / delta_n: the score mask and normalised score mask at the action (:393-394).  The
 // visited-set slot `tv` at `slot` of `tab` was requested by the caller (k0 / k1: the Zobrist key after the flip).  Shared
-// by the int8 kernel below and the fp64-field kernel of weighted graphs (weighted.cu).
+// by the int8 steps (env_step_group below, env_step_ring_kernel) and the fp64-field kernel of weighted graphs (weighted.cu).
 struct StepScalars {
     double score, nscore, best_score, best_nscore, rew;
     int n_visited;
@@ -169,7 +169,7 @@ __device__ __forceinline__ void env_step_group(const eco_graphs_t& g, const eco_
     j.v = make_uint2(0, 0);
     if (has && active) j.v = *reinterpret_cast<const uint2*>(g.J + ((size_t)gi * NP + a) * NP + lane * 8);
     const double mlr = g.gscal[(size_t)gi * 4 + 0];
-    const bool use_tab = (g.reserved & 1) != 0;       // couplings in {-1,0,1}: |gain| <= degree < NP
+    const bool use_tab = (g.reserved & ECO_GRAPHS_PM1) != 0;       // couplings in {-1,0,1}: |gain| <= degree < NP
     const float* gtab = g.gain_tab + (size_t)gi * tab_stride(NP) + NP;
     double qn = 1.0;
     ulonglong2 zob = make_ulonglong2(0, 0);

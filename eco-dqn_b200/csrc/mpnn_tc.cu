@@ -1200,7 +1200,7 @@ mpnn_tc_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const int3
 
 }  // namespace
 
-bool mpnn_tc_supported(const eco_graphs_t* g) { return g->N <= NPMAX && (g->reserved & 1) && g->tc_ops != nullptr; }
+bool mpnn_tc_supported(const eco_graphs_t* g) { return g->N <= NPMAX && (g->reserved & ECO_GRAPHS_PM1) && g->tc_ops != nullptr; }
 size_t mpnn_tc_scratch_bytes(int, int) { return (NWARPS + ISSUERS) * 1024 * 8 + 256; }   // room for the optional debug timeline
 size_t mpnn_tc_packed_bytes() { return (size_t)PK_WORDS * 4; }
 

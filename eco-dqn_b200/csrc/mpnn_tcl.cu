@@ -140,7 +140,7 @@ graph_aggregate_kernel(const eco_graphs_t g, const int32_t* __restrict__ graph_i
 
 }  // namespace
 
-bool mpnn_tcl_supported(const eco_graphs_t* g) { return (g->reserved & 1) && g->tc_ops != nullptr; }
+bool mpnn_tcl_supported(const eco_graphs_t* g) { return (g->reserved & ECO_GRAPHS_PM1) && g->tc_ops != nullptr; }
 
 // OUT = scale / deg * (X1 * IMG[which1] (+ X2 * IMG[which2]));  X*, OUT: [B][*][64] fp32 with the given episode strides
 int launch_tcl_contract(const eco_graphs_t* g, const int32_t* gidx, int B, const float* X1, int which1, const float* X2,

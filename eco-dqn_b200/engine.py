@@ -162,8 +162,8 @@ class GraphSet:
             stat = self.gstat.cpu().numpy()
         self.max_degree = int(stat[:, 0].max())
         self.pm1_only = not bool((stat[:, 3] & 1).any())
-        # bit0: couplings in {-1,0,1} -> tcgen05 MPNN path allowed
-        self.c.reserved = (1 if self.pm1_only else 0) | (_lib.GRAPHS_MIN_CUT if self.min_cut else 0)
+        # couplings in {-1,0,1} -> tcgen05 MPNN path allowed
+        self.c.reserved = (_lib.GRAPHS_PM1 if self.pm1_only else 0) | (_lib.GRAPHS_MIN_CUT if self.min_cut else 0)
         if validate:
             if (stat[:, 3] & 4).any():
                 raise ValueError("graph %d is not symmetric with a zero diagonal" % int(np.nonzero(stat[:, 3] & 4)[0][0]))

@@ -45,8 +45,9 @@ extern "C" {
 #define ECO_POLICY_NETWORK     1   /* argmax_i Q_i, lowest index on ties (experiments/utils.py:57-66)      */
 #define ECO_POLICY_GREEDY      2   /* argmax_i s_i h_i, stop when the best gain < 0 (src/agents/solver.py:105-131) */
 
-/* eco_graphs_t.reserved bit: OptimisationTarget.MIN_CUT instead of CUT (quality = qn - cut, qn = |sum of negative weights|,
- * masks = negated cut changes) */
+/* eco_graphs_t.reserved bits: every coupling is in {-1,0,1} (asserted by the caller, see gstat flags); OptimisationTarget.MIN_CUT
+ * instead of CUT (quality = qn - cut, qn = |sum of negative weights|, masks = negated cut changes) */
+#define ECO_GRAPHS_PM1         1
 #define ECO_GRAPHS_MIN_CUT     2
 
 /* eco_env_t.reserved mode bits: the S2V-DQN configuration of the reference (experiments/pretrained_agent/test_s2v.py) is
@@ -71,7 +72,7 @@ int         eco_abi_version(void);
  * of MaximumCutUnbiasedScorer (src/envs/score_solver.py:347-375): mlr, qn, lb.
  * --------------------------------------------------------------------------------------------------------- */
 typedef struct {
-    int32_t  G, N, NP, reserved;   /* reserved bit0: caller asserts every coupling is in {-1,0,1} (see gstat flags);
+    int32_t  G, N, NP, reserved;   /* ECO_GRAPHS_PM1: caller asserts every coupling is in {-1,0,1} (see gstat flags);
                                       ECO_GRAPHS_MIN_CUT: set BEFORE upload/load/update -- the constants below are the
                                       Min-Cut scorer's (score_solver.py:423-505) and every env kernel negates its masks */
     int8_t*  J;          /* [G, NP, NP]  couplings, zero padded                                              */

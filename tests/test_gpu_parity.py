@@ -300,7 +300,8 @@ def test_env_step_staged_ring_matches_subwarp_kernel(eng, n, variant):
     """B >= 4096 with caller-supplied actions runs env_step_ring_kernel (persistent warps, async-copy ring); smaller batches
     run the sub-warp kernel that the oracle tests pin.  Same episodes, same actions (out-of-range ones included): every
     state array, observation, reward and done flag must be identical.  "fast": the rollout configuration (+-1 couplings,
-    T + 1 <= 1024: the stripped vertex loop); "weights": couplings in -3 .. 3 and "long": T = 1100, both through the general loop."""
+    T + 1 <= 1024: the FAST instantiation); "weights": couplings in -3 .. 3 and "long": T = 1100, both through the general
+    instantiation."""
     rng = np.random.default_rng(1000 + n)
     B, G, T, steps = 4096 + 37, 5, 24, 24       # T small: episodes finish inside the test, done episodes stay untouched
     if variant == "long":
