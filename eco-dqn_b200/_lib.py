@@ -15,6 +15,7 @@ ENV_IRREVERSIBLE, ENV_DENSE_REWARD = 1, 2      # eco_env_t.reserved mode bits (i
 GRAPHS_PM1 = 1                                  # eco_graphs_t.reserved: every coupling in {-1,0,1}
 GRAPHS_MIN_CUT = 2                              # eco_graphs_t.reserved: OptimisationTarget.MIN_CUT
 MAX_SPINS = 2048
+MAX_SPINS_SPARSE = 32768                        # CSR graph sets (eco_sgraphs_t)
 
 vp = C.c_void_p
 i32 = C.c_int32
@@ -56,6 +57,14 @@ class WEnv(C.Structure):
 
 
 WGRAPH_NO_DEGREE, WGRAPH_ASYMMETRIC, WGRAPH_NONFINITE = 2, 4, 8   # eco_wgraphs_t.gstat flags
+
+
+class SGraphs(C.Structure):
+    _fields_ = [("G", i32), ("N", i32), ("NP", i32), ("reserved", i32), ("nnz", C.c_int64),
+                ("row_ptr", vp), ("col", vp), ("val", vp), ("gscal", vp), ("deg", vp), ("gstat", vp), ("dmax", vp)]
+
+
+SGRAPH_FIELD_RANGE, SGRAPH_NONCANONICAL = 8, 16                  # eco_sgraphs_t.gstat flags (besides 1, 2, 4)
 
 
 class Mpnn(C.Structure):
@@ -127,6 +136,16 @@ def lib():
         "eco_wmpnn_forward": (C.c_int, [P(WGraphs), P(Mpnn), i32, vp, vp, vp, C.c_float, vp, vp, vp, i32, vp]),
         "eco_wrollout": (C.c_int, [P(WGraphs), P(WEnv), P(Mpnn), i32, i32, C.c_float, vp, vp, i32, vp, vp, vp, vp]),
         "eco_wenv_results": (C.c_int, [P(WEnv), vp, vp, vp, vp]),
+        "eco_sgraphs_workspace_bytes": (C.c_size_t, [i32, i32, C.c_int64]),
+        "eco_sgraphs_bind": (C.c_int, [P(SGraphs), vp, i32, i32, C.c_int64]),
+        "eco_sgraphs_load_dev": (C.c_int, [P(SGraphs), vp, vp, vp, vp]),
+        "eco_senv_workspace_bytes": (C.c_size_t, [i32, i32, i32]),
+        "eco_senv_bind": (C.c_int, [P(Env), vp, i32, i32, i32, C.c_double]),
+        "eco_senv_reset": (C.c_int, [P(SGraphs), P(Env), vp, vp, vp]),
+        "eco_senv_step": (C.c_int, [P(SGraphs), P(Env), i32, vp, vp, vp, vp, vp, vp, vp]),
+        "eco_smpnn_scratch_bytes": (C.c_size_t, [i32, i32]),
+        "eco_smpnn_forward": (C.c_int, [P(SGraphs), P(Mpnn), i32, vp, vp, vp, C.c_float, vp, vp, vp, vp]),
+        "eco_srollout": (C.c_int, [P(SGraphs), P(Env), P(Mpnn), i32, i32, C.c_float, vp, vp, vp, vp, vp, vp]),
         "eco_session_create": (C.c_int, [P(vp), i32, i32, i32, i32, C.c_double, P(vp), i32]),
         "eco_session_destroy": (None, [vp]),
         "eco_session_rollout": (C.c_int, [vp, vp, vp, vp, i32, C.c_float, vp, vp, vp]),
@@ -146,7 +165,9 @@ EXPORTED = ["eco_last_error", "eco_abi_version", "eco_launch_count", "eco_profil
             "eco_mpnn_pack", "eco_mpnn_forward", "eco_rollout", "eco_session_create", "eco_session_destroy",
             "eco_session_rollout", "eco_wgraphs_workspace_bytes", "eco_wgraphs_bind", "eco_wgraphs_load_dev",
             "eco_wenv_workspace_bytes", "eco_wenv_bind", "eco_wenv_reset", "eco_wenv_step", "eco_wmpnn_forward", "eco_wrollout",
-            "eco_wenv_results"]
+            "eco_wenv_results", "eco_sgraphs_workspace_bytes", "eco_sgraphs_bind", "eco_sgraphs_load_dev",
+            "eco_senv_workspace_bytes", "eco_senv_bind", "eco_senv_reset", "eco_senv_step", "eco_smpnn_scratch_bytes",
+            "eco_smpnn_forward", "eco_srollout"]
 
 
 def check(rc):

@@ -161,6 +161,9 @@ class DQN:
         if not all(engine.is_int8_graph(g) for g in first):
             raise NotImplementedError("DQN training with real-valued couplings (EdgeType.RANDOM) is not supported: the "
                                       "training kernels take integer couplings; weighted graphs run rollouts only")
+        if n > _lib.MAX_SPINS:
+            raise NotImplementedError("DQN training on graphs of more than %d vertices is not supported: the training kernels "
+                                      "take the dense layout; sparse (CSR) graph sets run rollouts only" % _lib.MAX_SPINS)
         ring = np.zeros((self._ring_size, n, n), dtype=np.int8)
         ring[:] = engine.graphs_to_int8(first[0])[0]          # placeholder so that every slot holds a valid graph
         self._graphs = engine.GraphSet(ring, device=self.device, min_cut=self.min_cut)

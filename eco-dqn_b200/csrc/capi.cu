@@ -124,7 +124,20 @@ static void carve_wenv(eco_wenv_t* e, Carver& c, int B, int N, int T, double bas
     e->cut = c.take<double>((size_t)B * 2);
 }
 
+static void carve_sgraphs(eco_sgraphs_t* g, Carver& c, int G, int N, int64_t nnz) {
+    const int NP = padded_n(N);
+    g->G = G; g->N = N; g->NP = NP; g->reserved = 0; g->nnz = nnz;
+    g->row_ptr = c.take<int64_t>((size_t)G * N + 1);
+    g->col = c.take<int32_t>((size_t)nnz);
+    g->val = c.take<int8_t>((size_t)nnz);
+    g->gscal = c.take<double>((size_t)G * 4);
+    g->deg = c.take<float>((size_t)G * NP);
+    g->gstat = c.take<int32_t>((size_t)G * 4);
+    g->dmax = c.take<float>(64);
+}
+
 static bool shape_ok(int N) { return N >= 1 && N <= ECO_MAX_SPINS; }
+static bool sparse_shape_ok(int N) { return N >= 1 && N <= ECO_MAX_SPINS_SPARSE; }
 
 __global__ void frac_tab_kernel(float* tab, int N) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -608,6 +621,124 @@ int eco_wrollout(const eco_wgraphs_t* g, eco_wenv_t* env, const eco_mpnn_t* w, i
 int eco_wenv_results(const eco_wenv_t* env, double* best_cut, int8_t* best_spins, int32_t* steps, void* stream) {
     ECO_CHECK_ARG(env, ECO_ERR_INVALID, "eco_wenv_results: null argument");
     return launch_wenv_results(env, best_cut, best_spins, steps, (cudaStream_t)stream);
+}
+
+// ------------------------------------------------------------------------------------------------ sparse (CSR) graphs
+size_t eco_sgraphs_workspace_bytes(int32_t G, int32_t N, int64_t nnz) {
+    if (G < 1 || !sparse_shape_ok(N) || nnz < 0) return 0;
+    eco_sgraphs_t g;
+    Carver c(nullptr);
+    carve_sgraphs(&g, c, G, N, nnz);
+    return c.off;
+}
+
+int eco_sgraphs_bind(eco_sgraphs_t* g, void* ws, int32_t G, int32_t N, int64_t nnz) {
+    ECO_CHECK_ARG(g && ws, ECO_ERR_INVALID, "eco_sgraphs_bind: null argument");
+    ECO_CHECK_ARG(G >= 1 && sparse_shape_ok(N) && nnz >= 0, ECO_ERR_INVALID,
+                  "eco_sgraphs_bind: need G >= 1, 1 <= N <= %d and nnz >= 0 (got G=%d N=%d nnz=%lld)", ECO_MAX_SPINS_SPARSE, G, N,
+                  (long long)nnz);
+    ECO_CHECK_ARG(((uintptr_t)ws & 255) == 0, ECO_ERR_INVALID, "eco_sgraphs_bind: workspace must be 256-byte aligned");
+    Carver c(ws);
+    carve_sgraphs(g, c, G, N, nnz);
+    return ECO_OK;
+}
+
+int eco_sgraphs_load_dev(eco_sgraphs_t* g, const int64_t* row_ptr, const int32_t* col, const int8_t* val, void* stream) {
+    ECO_CHECK_ARG(g && g->row_ptr && row_ptr && (g->nnz == 0 || (col && val)), ECO_ERR_INVALID, "eco_sgraphs_load_dev: null argument");
+    ECO_CHECK_ARG(!(g->reserved & ECO_GRAPHS_MIN_CUT), ECO_ERR_UNSUPPORTED,
+                  "eco_sgraphs_load_dev: sparse graph sets support OptimisationTarget.CUT only");
+    cudaStream_t st = (cudaStream_t)stream;
+    ECO_CUDA(cudaMemcpyAsync(g->row_ptr, row_ptr, ((size_t)g->G * g->N + 1) * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+    if (g->nnz > 0) {
+        ECO_CUDA(cudaMemcpyAsync(g->col, col, (size_t)g->nnz * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+        ECO_CUDA(cudaMemcpyAsync(g->val, val, (size_t)g->nnz, cudaMemcpyDeviceToDevice, st));
+    }
+    return launch_sgraph_prepare(g, st);
+}
+
+size_t eco_senv_workspace_bytes(int32_t B, int32_t N, int32_t T) {
+    if (B < 1 || !sparse_shape_ok(N) || T < 1 || T > 65535) return 0;
+    eco_env_t e;
+    Carver c(nullptr);
+    carve_env(&e, c, B, N, T, 1.0);
+    return c.off;
+}
+
+int eco_senv_bind(eco_env_t* env, void* ws, int32_t B, int32_t N, int32_t T, double basin_reward) {
+    ECO_CHECK_ARG(env && ws, ECO_ERR_INVALID, "eco_senv_bind: null argument");
+    ECO_CHECK_ARG(B >= 1 && sparse_shape_ok(N), ECO_ERR_INVALID, "eco_senv_bind: need B >= 1 and 1 <= N <= %d",
+                  ECO_MAX_SPINS_SPARSE);
+    ECO_CHECK_ARG(T >= 1 && T <= 65535, ECO_ERR_INVALID, "eco_senv_bind: max_steps must be in [1, 65535] (got %d)", T);
+    ECO_CHECK_ARG(((uintptr_t)ws & 255) == 0, ECO_ERR_INVALID, "eco_senv_bind: workspace must be 256-byte aligned");
+    Carver c(ws);
+    carve_env(env, c, B, N, T, basin_reward);
+    return ECO_OK;
+}
+
+static int check_spair(const eco_sgraphs_t* g, const eco_env_t* env, const char* who) {
+    ECO_CHECK_ARG(g && env, ECO_ERR_INVALID, "%s: null argument", who);
+    ECO_CHECK_ARG(g->N == env->N && g->NP == env->NP, ECO_ERR_INVALID, "%s: graph set has N=%d but env has N=%d", who, g->N,
+                  env->N);
+    ECO_CHECK_ARG(env->reserved == 0 && !(g->reserved & ECO_GRAPHS_MIN_CUT), ECO_ERR_UNSUPPORTED,
+                  "%s: sparse graph sets support the ECO-DQN configuration only (CUT target, BLS reward, reversible spins)", who);
+    return ECO_OK;
+}
+
+int eco_senv_reset(const eco_sgraphs_t* g, eco_env_t* env, const int32_t* gidx, const int8_t* spins, void* stream) {
+    int rc = check_spair(g, env, "eco_senv_reset");
+    if (rc) return rc;
+    ECO_CHECK_ARG(gidx && spins, ECO_ERR_INVALID, "eco_senv_reset: null argument");
+    return launch_senv_reset(g, env, gidx, spins, (cudaStream_t)stream);
+}
+
+int eco_senv_step(const eco_sgraphs_t* g, eco_env_t* env, int32_t policy, const int32_t* actions, double* reward, uint8_t* done,
+                  int32_t* ha, double* hr, double* hs, void* stream) {
+    int rc = check_spair(g, env, "eco_senv_step");
+    if (rc) return rc;
+    ECO_CHECK_ARG(policy == ECO_POLICY_ACTIONS || policy == ECO_POLICY_GREEDY, ECO_ERR_INVALID,
+                  "eco_senv_step: policy must be ECO_POLICY_ACTIONS or ECO_POLICY_GREEDY");
+    ECO_CHECK_ARG(policy != ECO_POLICY_ACTIONS || actions, ECO_ERR_INVALID, "eco_senv_step: actions_dev is NULL");
+    return launch_senv_step(g, env, policy, actions, reward, done, ha, hr, hs, (cudaStream_t)stream);
+}
+
+size_t eco_smpnn_scratch_bytes(int32_t B, int32_t N) {
+    if (B < 1 || !sparse_shape_ok(N)) return 0;
+    return smpnn_scratch_bytes(B, N);
+}
+
+int eco_smpnn_forward(const eco_sgraphs_t* g, const eco_mpnn_t* w, int32_t B, const int32_t* gidx, const float* xn,
+                      const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, void* stream) {
+    ECO_CHECK_ARG(g && gidx && xn && xg && scratch, ECO_ERR_INVALID, "eco_smpnn_forward: null argument");
+    ECO_CHECK_ARG(B >= 1, ECO_ERR_INVALID, "eco_smpnn_forward: B must be >= 1");
+    ECO_CHECK_ARG(((uintptr_t)scratch & 15) == 0, ECO_ERR_INVALID, "eco_smpnn_forward: scratch must be 16-byte aligned");
+    int rc = check_weights(w, "eco_smpnn_forward");
+    if (rc) return rc;
+    return launch_smpnn(g, w, B, gidx, xn, xg, norm_max, q, actions, scratch, (cudaStream_t)stream);
+}
+
+int eco_srollout(const eco_sgraphs_t* g, eco_env_t* env, const eco_mpnn_t* w, int32_t n_steps, int32_t policy, float norm_max,
+                 int32_t* act, void* scratch, int32_t* ha, double* hr, double* hs, void* stream) {
+    int rc = check_spair(g, env, "eco_srollout");
+    if (rc) return rc;
+    ECO_CHECK_ARG(n_steps >= 0, ECO_ERR_INVALID, "eco_srollout: n_steps < 0");
+    ECO_CHECK_ARG(policy == ECO_POLICY_NETWORK || policy == ECO_POLICY_GREEDY, ECO_ERR_INVALID,
+                  "eco_srollout: policy must be ECO_POLICY_NETWORK or ECO_POLICY_GREEDY");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (policy == ECO_POLICY_GREEDY) {
+        for (int t = 0; t < n_steps; ++t) {
+            rc = launch_senv_step(g, env, ECO_POLICY_GREEDY, nullptr, nullptr, nullptr, ha, hr, hs, st);
+            if (rc) return rc;
+        }
+        return ECO_OK;
+    }
+    ECO_CHECK_ARG(act && scratch, ECO_ERR_INVALID, "eco_srollout: network policy needs actions and mpnn scratch buffers");
+    for (int t = 0; t < n_steps; ++t) {
+        rc = eco_smpnn_forward(g, w, env->B, env->graph_idx, env->xn, env->xg, norm_max, nullptr, act, scratch, stream);
+        if (rc) return rc;
+        rc = launch_senv_step(g, env, ECO_POLICY_ACTIONS, act, nullptr, nullptr, ha, hr, hs, st);
+        if (rc) return rc;
+    }
+    return ECO_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ session

@@ -132,6 +132,13 @@ int launch_wenv_results(const eco_wenv_t* we, double* best_cut, int8_t* best_spi
 int launch_mpnn_simt_w(const eco_wgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
                        const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);
 size_t mpnn_simt_scratch_bytes(int B, int N);
+int launch_sgraph_prepare(const eco_sgraphs_t* g, cudaStream_t st);
+int launch_senv_reset(const eco_sgraphs_t* g, eco_env_t* env, const int32_t* gidx, const int8_t* spins, cudaStream_t st);
+int launch_senv_step(const eco_sgraphs_t* g, eco_env_t* env, int policy, const int32_t* actions, double* reward, uint8_t* done,
+                     int32_t* ha, double* hr, double* hs, cudaStream_t st);
+size_t smpnn_scratch_bytes(int B, int N);
+int launch_smpnn(const eco_sgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn, const float* xg,
+                 float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);
 int launch_mpnn_tc(const eco_graphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
                    const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);
 bool mpnn_tc_can_fuse(const eco_graphs_t* g, const eco_env_t* env);

@@ -5,6 +5,7 @@ Host-side mirror of the reference's environment/agent surface for the rollout ho
   GraphSet             <- SingleGraphGenerator / SetGraphGenerator payloads (src/envs/utils.py:319-382) +
                           MaximumCutUnbiasedScorer constants (src/envs/score_solver.py:347-375)
   WeightedGraphSet     <- the same for real-valued couplings (EdgeType.RANDOM): fp64 environment, fp32(J) MPNN
+  SparseGraphSet       <- the same for integer couplings stored as CSR, up to 32 768 vertices (GSet G55 and up)
   BatchedSpinSystem    <- B x SpinSystemBase (src/envs/spinsystem.py:50-607): reset / step / observation /
                           best_* trackers, struct-of-arrays on the device
   MPNNWeights          <- MPNN.state_dict() (src/networks/mpnn.py:5-32; SURVEY.md appendix A.3)
@@ -16,7 +17,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import Graphs, Env, Mpnn, WGraphs, WEnv, check, lib
+from ._lib import Graphs, Env, Mpnn, SGraphs, WGraphs, WEnv, check, lib
 
 STATE_DICT_KEYS = (
     "node_init_embedding_layer.0.weight",
@@ -278,6 +279,123 @@ class WeightedGraphSet:
         return self.gscal[:, 2]
 
 
+def sparse_csr(n_vertices, graphs):
+    """Host canonicalisation of SparseGraphSet's input -> (row_ptr int64 [G*N + 1], col int32 [nnz], val int8 [nnz]).
+
+    Each entry of `graphs` is a `(rows, cols, weights)` triple -- every undirected edge once, as `read_mc_instance` returns
+    them; both directions are stored --, a scipy sparse matrix (every stored entry, as is) or a dense array (its non-zeros).
+    Duplicates resolve last-writer-wins, as in `eco_graphs_load_edges_dev` (the reference's `matrix[i, j] = w`); entries
+    whose final value is zero are dropped; columns are ascending within every row."""
+    import scipy.sparse as sps
+    n = int(n_vertices)
+    if n < 1 or n > _lib.MAX_SPINS_SPARSE:
+        raise ValueError("N=%d outside [1, ECO_MAX_SPINS_SPARSE=%d]" % (n, _lib.MAX_SPINS_SPARSE))
+    counts, cols, vals = [], [], []
+    for gph in graphs:
+        if sps.issparse(gph):
+            coo = gph.tocoo()
+            if coo.shape != (n, n):
+                raise ValueError("sparse matrix of shape %s in a set of %d-vertex graphs" % (coo.shape, n))
+            r, c, w = np.asarray(coo.row, dtype=np.int64), np.asarray(coo.col, dtype=np.int64), np.asarray(coo.data)
+        elif isinstance(gph, tuple) and len(gph) == 3:
+            r0, c0, w0 = (np.asarray(x).ravel() for x in gph)
+            if not (len(r0) == len(c0) == len(w0)):
+                raise ValueError("rows, cols and weights must have the same length")
+            # (i, j, w) then (j, i, w) for every edge, in input order: the later writer of a position wins
+            r = np.stack([r0, c0], axis=1).ravel().astype(np.int64)
+            c = np.stack([c0, r0], axis=1).ravel().astype(np.int64)
+            w = np.repeat(w0, 2)
+        else:
+            arr = np.asarray(gph)
+            if arr.shape != (n, n):
+                raise ValueError("dense graph of shape %s in a set of %d-vertex graphs" % (arr.shape, n))
+            r, c = np.nonzero(arr)
+            w = arr[r, c]
+        if w.size and (not np.issubdtype(w.dtype, np.number) or not np.isfinite(w).all() or
+                       (np.rint(w) != w).any() or np.abs(w).max() > 127):
+            raise NotImplementedError("sparse graph sets take integer couplings in [-127, 127]; real-valued graphs of more "
+                                      "than %d vertices are not supported" % _lib.MAX_SPINS)
+        if w.size and (r.min() < 0 or c.min() < 0 or r.max() >= n or c.max() >= n):
+            raise ValueError("an entry names a vertex outside [0, %d)" % n)
+        key = r * n + c
+        # last occurrence of every position: first occurrence in the reversed order; np.unique sorts the keys (row, col)
+        ukey, first_rev = np.unique(key[::-1], return_index=True)
+        uval = w[::-1][first_rev]
+        keep = uval != 0
+        ukey, uval = ukey[keep], uval[keep]
+        counts.append(np.bincount(ukey // n, minlength=n))
+        cols.append((ukey % n).astype(np.int32))
+        vals.append(np.rint(uval).astype(np.int8))
+    if not counts:
+        raise ValueError("empty graph set")
+    row_ptr = np.zeros(len(counts) * n + 1, dtype=np.int64)
+    np.cumsum(np.concatenate(counts), out=row_ptr[1:])
+    return row_ptr, np.concatenate(cols), np.concatenate(vals)
+
+
+class SparseGraphSet:
+    """G integer-weight graphs of up to ECO_MAX_SPINS_SPARSE (32 768) vertices stored as CSR on the device: the GSet instances
+    (G55 and up) that the dense N x N layout of GraphSet cannot hold.  The host canonicalises the input (sparse_csr) and
+    uploads row_ptr / col / val only; the device computes the scorer constants, the degrees and the validity flags.
+    ECO-DQN rollout configuration (CUT target) and the Greedy baseline.  Any N >= 1 is accepted (for N <= 2048 every
+    result equals GraphSet's)."""
+    weighted = False
+    sparse = True
+    min_cut = False
+
+    def __init__(self, n_vertices, graphs, device=None, validate=True, min_cut=False):
+        if min_cut:
+            raise NotImplementedError("OptimisationTarget.MIN_CUT is not supported on sparse graph sets (CUT target only)")
+        self.device = _require_cuda(device)
+        row_ptr, col, val = sparse_csr(n_vertices, graphs)
+        self.N = int(n_vertices)
+        self.G = (len(row_ptr) - 1) // self.N
+        self.nnz = int(row_ptr[-1])
+        L = lib()
+        with torch.cuda.device(self.device):
+            self._ws = torch.zeros(L.eco_sgraphs_workspace_bytes(self.G, self.N, self.nnz), dtype=torch.uint8, device=self.device)
+            self.c = SGraphs()
+            check(L.eco_sgraphs_bind(C.byref(self.c), _ptr(self._ws), self.G, self.N, self.nnz))
+            dev = [torch.from_numpy(np.ascontiguousarray(x)).to(self.device) for x in (row_ptr, col, val)]
+            check(L.eco_sgraphs_load_dev(C.byref(self.c), _ptr(dev[0]), _ptr(dev[1]), _ptr(dev[2]), _stream()))
+            self.NP = int(self.c.NP)
+            G, NP, nnz = self.G, self.NP, self.nnz
+            self.row_ptr = _view(self._ws, self.c.row_ptr, G * self.N + 1, torch.int64, (G * self.N + 1,))
+            self.col = _view(self._ws, self.c.col, nnz, torch.int32, (nnz,))
+            self.val = _view(self._ws, self.c.val, nnz, torch.int8, (nnz,))
+            self.gscal = _view(self._ws, self.c.gscal, G * 4, torch.float64, (G, 4))
+            self.deg = _view(self._ws, self.c.deg, G * NP, torch.float32, (G, NP))
+            self.gstat = _view(self._ws, self.c.gstat, G * 4, torch.int32, (G, 4))
+            self.dmax = _view(self._ws, self.c.dmax, 1, torch.float32, (1,))
+            stat = self.gstat.cpu().numpy()
+        self.max_degree = int(stat[:, 0].max())
+        self.pm1_only = not bool((stat[:, 3] & 1).any())
+        self.c.reserved = _lib.GRAPHS_PM1 if self.pm1_only else 0
+        if validate:
+            first = lambda bit: int(np.nonzero(stat[:, 3] & bit)[0][0])
+            if (stat[:, 3] & _lib.SGRAPH_NONCANONICAL).any():
+                raise ValueError("graph %d is not canonical CSR" % first(_lib.SGRAPH_NONCANONICAL))
+            if (stat[:, 3] & 4).any():
+                raise ValueError("graph %d is not symmetric with a zero diagonal" % first(4))
+            if (stat[:, 3] & 2).any():
+                # the reference recurses forever on such a graph (spinsystem.py:209-211)
+                raise ValueError("graph %d has no non-zero weighted degree" % first(2))
+            if stat[:, 2].max() > 32767:
+                raise NotImplementedError("weighted degree exceeds the int16 local-field range")
+
+    @property
+    def mlr(self):
+        return self.gscal[:, 0]
+
+    @property
+    def qn(self):
+        return self.gscal[:, 1]
+
+    @property
+    def lb(self):
+        return self.gscal[:, 2]
+
+
 def graph_set(graphs, device=None, validate=True, min_cut=False):
     """GraphSet when every coupling is an integer in [-127, 127], WeightedGraphSet otherwise (what the drop-in surface
     routes through: integer graphs keep the int8 path and its results bit for bit)."""
@@ -362,6 +480,11 @@ class BatchedSpinSystem:
         if self.weighted and (not reversible_spins or dense_reward):
             raise NotImplementedError("irreversible spins / dense reward (S2V-DQN) with real-valued couplings are not "
                                       "supported: weighted graphs run the ECO-DQN configuration only")
+        # CSR graph sets: the int8 state (eco_env_t) stepped in O(degree), ECO-DQN configuration only
+        self.sparse = bool(getattr(graphset, "sparse", False))
+        if self.sparse and (not reversible_spins or dense_reward):
+            raise NotImplementedError("irreversible spins / dense reward (S2V-DQN) are not supported on sparse graph sets: "
+                                      "they run the ECO-DQN configuration only")
         self.basin_reward = basin_reward
         self.mpnn_impl = mpnn_impl
         L = lib()
@@ -373,6 +496,12 @@ class BatchedSpinSystem:
                 self.c = WEnv()
                 check(L.eco_wenv_bind(C.byref(self.c), _ptr(self._ws), self.B, self.N, self.T, basin))
                 self._base = self.c.base        # (shares the memory of self.c)
+            elif self.sparse:
+                nbytes = L.eco_senv_workspace_bytes(self.B, self.N, self.T)
+                self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
+                self.c = Env()
+                check(L.eco_senv_bind(C.byref(self.c), _ptr(self._ws), self.B, self.N, self.T, basin))
+                self._base = self.c
             else:
                 nbytes = L.eco_env_workspace_bytes(self.B, self.N, self.T)
                 self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
@@ -443,7 +572,7 @@ class BatchedSpinSystem:
             if int(gi.min()) < 0 or int(gi.max()) >= self.gs.G:
                 raise ValueError("graph_idx out of range")
         with torch.cuda.device(self.device):
-            reset = lib().eco_wenv_reset if self.weighted else lib().eco_env_reset
+            reset = lib().eco_wenv_reset if self.weighted else lib().eco_senv_reset if self.sparse else lib().eco_env_reset
             check(reset(C.byref(self.gs.c), C.byref(self.c), _ptr(gi), _ptr(sp), _stream()))
         self.current_step = 0
         self._is_reset = True
@@ -463,18 +592,21 @@ class BatchedSpinSystem:
         if a.shape != (self.B,):
             raise ValueError("actions must be [B]")
         ha, hr, hs = hist if hist is not None else (None, None, None)
-        step = lib().eco_wenv_step if self.weighted else lib().eco_env_step
+        step = self._step_fn()
         with torch.cuda.device(self.device):
             check(step(C.byref(self.gs.c), C.byref(self.c), _lib.POLICY_ACTIONS, _ptr(a),
                                      _ptr(self._reward), _ptr(self._done), _ptr(ha), _ptr(hr), _ptr(hs), _stream()))
         self.current_step += 1
         return self._reward, self._done
 
+    def _step_fn(self):
+        return lib().eco_wenv_step if self.weighted else lib().eco_senv_step if self.sparse else lib().eco_env_step
+
     def greedy_step(self, hist=None):
         """One step of the Greedy solver (src/agents/solver.py:105-131) for every episode still running."""
         self._check_steppable()
         ha, hr, hs = hist if hist is not None else (None, None, None)
-        step = lib().eco_wenv_step if self.weighted else lib().eco_env_step
+        step = self._step_fn()
         with torch.cuda.device(self.device):
             check(step(C.byref(self.gs.c), C.byref(self.c), _lib.POLICY_GREEDY, None,
                                      _ptr(self._reward), _ptr(self._done), _ptr(ha), _ptr(hr), _ptr(hs), _stream()))
@@ -483,7 +615,10 @@ class BatchedSpinSystem:
 
     # ------------------------------------------------------------------ Q-network
     def _scratch_for(self, B):
-        nb = lib().eco_mpnn_scratch_bytes(B, self.N, self.mpnn_impl)
+        if self.sparse:
+            nb = lib().eco_smpnn_scratch_bytes(B, self.N)
+        else:
+            nb = lib().eco_mpnn_scratch_bytes(B, self.N, self.mpnn_impl)
         if self._scratch is None or self._scratch.numel() < nb:
             self._scratch = torch.empty(nb, dtype=torch.uint8, device=self.device)
         return self._scratch
@@ -493,6 +628,15 @@ class BatchedSpinSystem:
         q = torch.zeros(self.B, self.NP, dtype=torch.float32, device=self.device)
         acts = self._actions if want_actions else None
         nm = float(norm_max) if norm_max is not None else 0.0
+        if self.sparse:
+            if (self.mpnn_impl if impl is None else impl) == _lib.MPNN_TCGEN05:
+                raise NotImplementedError("the tensor-core MPNN needs the dense layout; sparse graph sets run the CUDA-core "
+                                          "gather forward")
+            with torch.cuda.device(self.device):
+                check(lib().eco_smpnn_forward(C.byref(self.gs.c), C.byref(weights.c), self.B, _ptr(self.graph_idx),
+                                              _ptr(self.xn), _ptr(self.xg), nm, _ptr(q), _ptr(acts),
+                                              _ptr(self._scratch_for(self.B)), _stream()))
+            return q[:, :self.N], acts
         forward = lib().eco_wmpnn_forward if self.weighted else lib().eco_mpnn_forward
         with torch.cuda.device(self.device):
             check(forward(C.byref(self.gs.c), C.byref(weights.c), self.B, _ptr(self.graph_idx),
@@ -523,6 +667,15 @@ class BatchedSpinSystem:
         if pol == _lib.POLICY_NETWORK and weights is None:
             raise ValueError("network policy needs weights")
         nm = float(norm_max) if norm_max is not None else -1.0
+        if self.sparse:
+            with torch.cuda.device(self.device):
+                check(lib().eco_srollout(C.byref(self.gs.c), C.byref(self.c),
+                                         C.byref(weights.c) if weights is not None else None, n_steps, pol, nm,
+                                         _ptr(self._actions),
+                                         _ptr(self._scratch_for(self.B)) if pol == _lib.POLICY_NETWORK else None,
+                                         _ptr(hist[0]), _ptr(hist[1]), _ptr(hist[2]), _stream()))
+            self.current_step += n_steps
+            return hist if record_history else None
         rollout = lib().eco_wrollout if self.weighted else lib().eco_rollout
         with torch.cuda.device(self.device):
             check(rollout(C.byref(self.gs.c), C.byref(self.c),
@@ -572,6 +725,9 @@ class HostSession:
 
     def __init__(self, G, N, B, T, basin_reward, state_dict, impl=_lib.MPNN_AUTO):
         _require_cuda()
+        if N > _lib.MAX_SPINS:
+            raise NotImplementedError("HostSession takes the dense layout (N <= %d); larger graphs run through SparseGraphSet + "
+                                      "BatchedSpinSystem" % _lib.MAX_SPINS)
         self.G, self.N, self.B, self.T = G, N, B, T
         self._w = [np.ascontiguousarray(np.asarray(state_dict[k].cpu() if torch.is_tensor(state_dict[k])
                                                    else state_dict[k], dtype=np.float32)) for k in STATE_DICT_KEYS]

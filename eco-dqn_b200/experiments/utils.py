@@ -80,9 +80,13 @@ def test_network(network, env_args, graphs_test, device=None, step_factor=1, bat
     for n, idxs in groups.items():
         n_steps = int(n * step_factor)
         args = _check_env_args(env_args, n_steps)
-        # integer couplings in [-127, 127]: the int8 path; anything else (EdgeType.RANDOM): the fp64 weighted path
-        gs = engine.graph_set(np.stack([graphs_test[j] for j in idxs]), device=dev,
-                              min_cut=args["optimisation_target"] == OptimisationTarget.MIN_CUT)
+        min_cut = args["optimisation_target"] == OptimisationTarget.MIN_CUT
+        if n > engine._lib.MAX_SPINS:
+            # more vertices than the dense layout holds: integer couplings as CSR (real-valued ones raise)
+            gs = engine.SparseGraphSet(n, [graphs_test[j] for j in idxs], device=dev, min_cut=min_cut)
+        else:
+            # integer couplings in [-127, 127]: the int8 path; anything else (EdgeType.RANDOM): the fp64 weighted path
+            gs = engine.graph_set(np.stack([graphs_test[j] for j in idxs]), device=dev, min_cut=min_cut)
         G = len(idxs)
         B = G * n_attempts
         gidx = np.repeat(np.arange(G, dtype=np.int32), n_attempts)
@@ -212,13 +216,32 @@ def load_graph_set(graph_save_loc):
     return graphs_test
 
 
+def _n_of(g):
+    return g.number_of_nodes() if isinstance(g, nx.Graph) else g.shape[0]
+
+
+def _sparse_adjacency(g):
+    """One pickled graph for SparseGraphSet without an N x N host matrix: scipy matrices as they are, networkx graphs through
+    their sparse adjacency (the entries of `nx.to_numpy_array`: edge attribute `weight`, default 1, same vertex order),
+    anything else as its dense array."""
+    if isinstance(g, nx.Graph):
+        return nx.to_scipy_sparse_array(g, weight="weight", format="coo")
+    return g
+
+
 def load_graph_set_device(graph_save_loc, device=None, min_cut=False):
     """The same pickle straight into an engine.GraphSet (all graphs of the file must share N, as the reference's batched
     tester assumes per graph anyway).  A file of scipy sparse matrices (the csr pickles) goes through the sparse ingest --
     only the stored entries cross PCIe, the dense int8 couplings are built on the device; anything else is uploaded as int8,
-    or, when a coupling is not an integer in [-127, 127], as an fp64 engine.WeightedGraphSet."""
+    or, when a coupling is not an integer in [-127, 127], as an fp64 engine.WeightedGraphSet.  Graphs of more than 2048
+    vertices become an engine.SparseGraphSet (CSR on the device)."""
     with open(graph_save_loc, 'rb') as f:
         raw = pickle.load(f)
+    if len(raw) and _n_of(raw[0]) > engine._lib.MAX_SPINS:
+        if min_cut:
+            raise NotImplementedError("OptimisationTarget.MIN_CUT is not supported on sparse graph sets (CUT target only)")
+        n = _n_of(raw[0])
+        return engine.SparseGraphSet(n, [_sparse_adjacency(g) for g in raw], device=device)
     if len(raw) and all(sp.sparse.issparse(g) for g in raw):
         return engine.GraphSet.from_edges(raw[0].shape[0], raw, device=device, min_cut=min_cut)
     graphs = [to_dense_adjacency(g) for g in raw]
@@ -228,11 +251,14 @@ def load_graph_set_device(graph_save_loc, device=None, min_cut=False):
 def load_mc_instances_device(graph_dir, graph_names, device=None, min_cut=False):
     """GSet `.mc` instances (all of one size) straight into an engine.GraphSet through the sparse ingest: the edge lists go to
     the device (5 bytes per edge) and the dense int8 couplings are built there -- no N x N float64 matrix, which is what
-    `load_graph` (reference experiments/utils.py:391-418) builds per instance."""
+    `load_graph` (reference experiments/utils.py:391-418) builds per instance.  Instances of more than 2048 vertices (G55 and
+    up) become an engine.SparseGraphSet: the same edge lists, kept as CSR on the device."""
     insts = [read_mc_instance(os.path.join(graph_dir, 'instances', name + '.mc')) for name in graph_names]
     n = insts[0][0]
     if any(i[0] != n for i in insts):
         raise ValueError("all instances of one GraphSet must have the same number of vertices")
+    if n > engine._lib.MAX_SPINS:
+        return engine.SparseGraphSet(n, [(r, c, w) for _, _, r, c, w in insts], device=device, min_cut=min_cut)
     return engine.GraphSet.from_edges(n, [(r, c, w) for _, _, r, c, w in insts], device=device, min_cut=min_cut)
 
 

@@ -17,7 +17,8 @@
  *   - Vertices are padded to NP = 16*ceil(N/16) per row; padded entries are zero and never selected.
  *   - Integer-weight graphs (int8 couplings; the reference's EdgeType.UNIFORM / DISCRETE) through eco_graphs_t, and
  *     real-valued graphs (fp64 couplings; EdgeType.RANDOM) through the eco_wgraphs_t / eco_wenv_t entry points at the
- *     end of this header.  There is no CPU fallback anywhere in this library.
+ *     end of this header, and integer-weight graphs of up to ECO_MAX_SPINS_SPARSE vertices stored as CSR through the
+ *     eco_sgraphs_t entry points after them.  There is no CPU fallback anywhere in this library.
  */
 #ifndef ECODQN_B200_H
 #define ECODQN_B200_H
@@ -390,6 +391,63 @@ int    eco_wrollout(const eco_wgraphs_t* g, eco_wenv_t* env, const eco_mpnn_t* w
 /* best cut (fp64), best spins [B, N] int8, step count.  Any may be NULL. */
 int    eco_wenv_results(const eco_wenv_t* env, double* best_cut_dev, int8_t* best_spins_dev, int32_t* steps_dev,
                         void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------
+ * Sparse graph sets: G graphs of up to ECO_MAX_SPINS_SPARSE vertices stored as CSR, integer couplings in [-127, 127] -- the
+ * GSet instances (G55: 5000 vertices, G70 / G72: 10 000, G81: 20 000) that the dense N x N layout cannot hold.  ECO-DQN
+ * rollout configuration (CUT target, BLS and basin reward, reversible spins, Stopping.NORMAL) plus the Greedy baseline.
+ * The environment is a plain eco_env_t (same layout and integer / fp64 rules as the int8 path), so eco_env_set_tables,
+ * eco_env_observation, eco_env_best_spins and eco_env_results take it unchanged; for N <= ECO_MAX_SPINS every state array
+ * equals the dense path's bit for bit.  The step costs O(degree) plus one O(N) feature row (time since flip); the MPNN
+ * aggregates by gathering neighbour rows.  N is bounded by the uint16 last-flip steps with max_steps <= 65535 (the
+ * reference's test scripts run 2N steps).  MIN_CUT and the S2V-DQN env modes are ECO_ERR_UNSUPPORTED.
+ * --------------------------------------------------------------------------------------------------------- */
+#define ECO_MAX_SPINS_SPARSE     32768
+#define ECO_SGRAPH_FIELD_RANGE   8    /* gstat flag: a row's sum of |couplings| exceeds 32767 (the int16 local fields)       */
+#define ECO_SGRAPH_NONCANONICAL  16   /* gstat flag: a row pointer, column or stored value breaks the CSR rules below        */
+
+typedef struct {
+    int32_t  G, N, NP, reserved;   /* reserved: ECO_GRAPHS_PM1 as for eco_graphs_t (informational); ECO_GRAPHS_MIN_CUT is not
+                                      supported                                                                             */
+    int64_t  nnz;        /* stored entries of all graphs                                                                */
+    int64_t* row_ptr;    /* [G*N + 1]    global offsets: row i of graph g is entries row_ptr[g*N + i] .. row_ptr[g*N + i + 1] - 1 */
+    int32_t* col;        /* [nnz]        column, strictly ascending within a row (every sum over a row has one fixed order)  */
+    int8_t*  val;        /* [nnz]        coupling, non-zero; both directions of every edge are stored                       */
+    double*  gscal;      /* [G, 4]       mlr, qn, lb, sum_ij J_ij (as eco_graphs_t)                                         */
+    float*   deg;        /* [G, NP]      max(1, non-zeros of row i)                                                         */
+    int32_t* gstat;      /* [G, 4]       max degree, nnz, max row sum of |J|, flags (eco_graphs_t meanings:
+                                         bit0 weights outside {-1,0,1}, bit1 all weighted degrees zero, bit2 not symmetric /
+                                         non-zero diagonal; plus ECO_SGRAPH_FIELD_RANGE, ECO_SGRAPH_NONCANONICAL)         */
+    float*   dmax;       /* [1]          max degree over the whole set                                                      */
+} eco_sgraphs_t;
+
+size_t eco_sgraphs_workspace_bytes(int32_t G, int32_t N, int64_t nnz);
+int    eco_sgraphs_bind(eco_sgraphs_t* g, void* workspace_dev, int32_t G, int32_t N, int64_t nnz);
+/* canonical CSR already on the device (row_ptr_dev [G*N + 1] int64 with row_ptr_dev[0] = 0 and row_ptr_dev[G*N] = nnz,
+ * col_dev [nnz] int32, val_dev [nnz] int8): copied into the workspace (async), then the constants and flags are computed */
+int    eco_sgraphs_load_dev(eco_sgraphs_t* g, const int64_t* row_ptr_dev, const int32_t* col_dev, const int8_t* val_dev,
+                            void* stream);
+
+/* an eco_env_t for 1 <= N <= ECO_MAX_SPINS_SPARSE (eco_env_workspace_bytes / eco_env_bind with the sparse size limit) */
+size_t eco_senv_workspace_bytes(int32_t B, int32_t N, int32_t T);
+int    eco_senv_bind(eco_env_t* env, void* workspace_dev, int32_t B, int32_t N, int32_t T, double basin_reward);
+/* reset / step: arguments, policies (ECO_POLICY_ACTIONS, ECO_POLICY_GREEDY) and history arrays as eco_env_reset / eco_env_step */
+int    eco_senv_reset(const eco_sgraphs_t* g, eco_env_t* env, const int32_t* graph_idx_dev, const int8_t* init_spins_dev,
+                      void* stream);
+int    eco_senv_step(const eco_sgraphs_t* g, eco_env_t* env, int32_t policy, const int32_t* actions_dev, double* reward_dev,
+                     uint8_t* done_dev, int32_t* hist_actions_dev, double* hist_rewards_dev, double* hist_scores_dev,
+                     void* stream);
+/* MPNN.forward (mpnn.py:40-159) + argmax on fp32 CUDA cores; arguments and norm_max modes as eco_mpnn_forward.
+ * scratch_dev >= eco_smpnn_scratch_bytes(B, N), 16-byte aligned. */
+size_t eco_smpnn_scratch_bytes(int32_t B, int32_t N);
+int    eco_smpnn_forward(const eco_sgraphs_t* g, const eco_mpnn_t* w, int32_t B, const int32_t* graph_idx_dev,
+                         const float* xn_dev, const float* xg_dev, float norm_max, float* q_dev, int32_t* actions_dev,
+                         void* scratch_dev, void* stream);
+/* rollout: ECO_POLICY_NETWORK (n_steps x [forward + argmax -> step]) or ECO_POLICY_GREEDY; arguments as eco_rollout,
+ * mpnn_scratch_dev sized by eco_smpnn_scratch_bytes */
+int    eco_srollout(const eco_sgraphs_t* g, eco_env_t* env, const eco_mpnn_t* w, int32_t n_steps, int32_t policy,
+                    float norm_max, int32_t* actions_scratch_dev, void* mpnn_scratch_dev, int32_t* hist_actions_dev,
+                    double* hist_rewards_dev, double* hist_scores_dev, void* stream);
 
 #ifdef __cplusplus
 }
