@@ -16,5 +16,7 @@ Modules
   spin_env.py  restates src/envs/spinsystem.py + score_solver.py (MaximumCutUnbiasedScorer) +
                utils.py (calculate_cut, calculate_cut_changes, HistoryBuffer)
   mpnn.py      restates src/networks/mpnn.py (forward only, fp32, as written: dense [B,N,N,63] edge stage)
+  mpnn64.py    the same forward in float64 over a CSR graph, explicit degrees and divisor, differentiable
+               (the reference the kernels' precision tests compare with)
   rollout.py   restates experiments/utils.py::__test_network_batched (greedy-Q loop, Greedy baseline)
 """
