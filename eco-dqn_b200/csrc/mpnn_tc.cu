@@ -36,7 +36,8 @@
 //                 its results.  Warp 19 works through the tail of the PREVIOUS episode (pooling, W_p, Q, argmax and, in a
 //                 rollout, SpinSystemBase.step for that episode; packed mode: the K episodes of the previous pack) while
 //                 the others are on the next one.
-//   rollout       FUSED: one launch per rollout -- every CTA takes its own episodes through all steps (see FusedEnv).
+//   rollout       FUSED: one launch per rollout -- every CTA takes its own episodes through all steps, two or three
+//                 episodes at a time (see FusedEnv).
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
@@ -235,9 +236,14 @@ __device__ __forceinline__ void issue_part(const Ctx& c, uint32_t acc_col, uint3
 // FUSED (rollouts of the ECO-DQN configuration): the warp that has just taken an episode's argmax also applies the flip --
 // SpinSystemBase.step for that episode (env_step_device.cuh), state and next observations written back -- and, because
 // episodes never interact, the CTA then simply carries on: it takes ITS episodes through all `n_steps` steps of the rollout
-// in one launch (item = (step, episode), step-major), with no grid-wide synchronisation at all.  An episode's next
+// in one launch, with no grid-wide synchronisation at all.  Its episode list is cut into windows of two consecutive entries
+// (the last window takes a third when the count is odd); a window goes through all steps, its members taking turns, before
+// the next window starts: item = (window, step, member).  So only the operand images of 2 - 3 episodes per CTA are live at
+// a time (148 CTAs x 3 x 173 kB <= 77 MB at N = 200: they stay in L2, and each is read from HBM once per rollout rather
+// than once per step, which a step-major order over 4096 distinct graphs = 708 MB of images would need).  An episode's next
 // observations are read (cp.async.cg: L2, never a stale L1 line) at least one whole item after the tail warp wrote and
-// fenced them, which needs >= 2 episodes per CTA (checked by the launcher).  A rollout is ONE launch instead of 2 T.
+// fenced them, which needs >= 2 members per window, i.e. >= 2 episodes per CTA (checked by the launcher).  A rollout is ONE
+// launch instead of 2 T.
 struct FusedEnv {
     eco_env_t env;
     int32_t* hist_a;
@@ -287,10 +293,17 @@ mpnn_tc_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const int3
     // padding columns of H^T / E^T stays finite (0 x NaN in an aggregation would poison real vertices).
     const int N8 = PACKED ? NP : ((N + 7) & ~7);
     const int npacks = (B + K - 1) / K;
-    // this CTA's work: episodes (packs) blockIdx.x, + gridDim.x, ...; FUSED: that list once per rollout step
+    // this CTA's work: episodes (packs) blockIdx.x, + gridDim.x, ...; FUSED: every entry of that list once per rollout step,
+    // window by window (see FusedEnv): item = (window, step, member)
     const int n_e = (int)blockIdx.x < npacks ? (npacks - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
     const int n_items = n_e * (FUSED ? fe.n_steps : 1);
-    auto item_ep = [&](int it) { return (int)blockIdx.x + (FUSED ? it % n_e : it) * (int)gridDim.x; };
+    auto item_ep = [&](int it) {
+        if (!FUSED) return (int)blockIdx.x + it * (int)gridDim.x;
+        const int nw = n_e >> 1, span = 2 * fe.n_steps;          // windows; items of a two-entry window
+        const int wi = min(it / span, nw - 1);                    // (the last window takes the odd entry: three members)
+        const int members = wi == nw - 1 ? n_e - 2 * wi : 2;
+        return (int)blockIdx.x + (2 * wi + (it - wi * span) % members) * (int)gridDim.x;
+    };
     auto vertex_ok = [&](int n) { return PACKED ? (n % NPs) < Ns : n < N; };     // not a padding vertex
     // PACKED extras live behind the (at most 192 x 192) adjacency image
     float* rdmaxv = reinterpret_cast<float*>(smem + SM_A + PACK_NPMAX * PACK_NPMAX * 2);   // [192] 1 / deg_max of the vertex's graph
@@ -758,6 +771,14 @@ mpnn_tc_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const int3
         }
     }
     if (c.warp < NWARPS && n_items > 0) {
+        {   // W_ef is the same for every item and its columns overlap no other TMEM range: stored once per launch
+            uint4 wef[32 / (8 * SUBS)];
+            ldg_weights<32>(c, pk + PK_WEF, wef);
+            sttm_weights<32>(c, wef, T_WEF);
+            tmem_st_wait();
+            tc_fence_before();
+            workers_sync();           // complete (all 16 warps' columns) before either group signals its issuer
+        }
         if (PACKED) load_inputs(blockIdx.x);
         else if (c.grp == 1) stage_inputs(blockIdx.x);
     }
@@ -877,8 +898,6 @@ mpnn_tc_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const int3
         cxa = fmaf(wxa[7], gl.w, cxa); cxb = fmaf(wxb[7], gl.w, cxb); cia = fmaf(wia[6], gl.w, cia); cib = fmaf(wib[6], gl.w, cib);
         if (PACKED) { cxa = 0.f; cxb = 0.f; cia = 0.f; cib = 0.f; }      // (all 7 observations come from xf)
         constexpr int NOBS = PACKED ? 7 : 3;
-        uint4 wef[32 / (8 * SUBS)];
-        ldg_weights<32>(c, pk + PK_WEF, wef);
         TL(2);
         if (PACKED) workers_sync();                       // xf visible
         TL(3);
@@ -916,7 +935,6 @@ mpnn_tc_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const int3
                 tmem_st_16x128b_x2(tmem_addr(c.tmem, 32 * c.q, T_D + 8 * blk), dh);
                 tmem_st_16x128b_x2(tmem_addr(c.tmem, 32 * c.q + 16, T_D + 8 * blk), dl);
                 }
-                if (r == 0) sttm_weights<32>(c, wef, T_WEF);
                 tmem_st_wait();                       // -> issuer: this warp's share of round r is in TMEM
                 tc_fence_before();
                 __syncwarp();
@@ -924,8 +942,6 @@ mpnn_tc_kernel(const eco_graphs_t g, const eco_mpnn_t w, const int B, const int3
             }
         }
         TL(4);
-        workers_sync();                               // W_ef (stored by all 16 warps) is complete before any group signals its issuer
-        TL(6);
         {   // layer-0 weights: L2 -> registers while the edge contraction runs, registers -> TMEM once S / D are dead
             uint4 wm[64 / (8 * SUBS)], wu[64 / (8 * SUBS)];
             ldg_weights<64>(c, pk + PK_WM, wm);
