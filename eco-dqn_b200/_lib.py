@@ -116,6 +116,10 @@ def lib():
         "eco_mpnn_grad_ev": (C.c_int, [P(Graphs), P(Mpnn), i32, vp, vp, vp, C.c_float, vp, vp, i32, vp, vp, vp, vp, vp]),
         "eco_mpnn_adam": (C.c_int, [P(Mpnn), vp, vp, vp, i32, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, vp]),
         "eco_mpnn_adam_dev": (C.c_int, [P(Mpnn), vp, vp, vp, vp, vp, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, vp]),
+        "eco_dqn_masked_td_target": (C.c_int, [i32, i32, i32, vp, vp, vp, vp, vp, C.c_float, i32, i32, vp, vp, vp]),
+        "eco_dqn_masked_argmax": (C.c_int, [i32, i32, i32, vp, vp, vp, vp]),
+        "eco_dqn_masked_explore": (C.c_int, [P(Env), vp, vp, vp, vp, vp, vp]),
+        "eco_mpnn_grad_obs": (C.c_int, [P(Graphs), P(Mpnn), i32, vp, vp, vp, C.c_float, vp, vp, i32, i32, vp, vp, vp, vp, vp]),
         "eco_dp_create": (C.c_int, [P(vp), i32, i32]),
         "eco_dp_handle": (C.c_int, [vp, vp]),
         "eco_dp_open": (C.c_int, [vp, vp]),
@@ -161,7 +165,7 @@ def lib():
 EXPORTED = ["eco_last_error", "eco_abi_version", "eco_launch_count", "eco_profile_enable", "eco_profile_read", "eco_graphs_workspace_bytes",
             "eco_graphs_bind", "eco_graphs_upload", "eco_graphs_load_dev", "eco_graphs_update", "eco_graphs_load_edges_dev", "eco_env_workspace_bytes",
             "eco_env_bind", "eco_env_set_tables", "eco_env_reset", "eco_env_step", "eco_env_observation",
-            "eco_env_best_spins", "eco_env_masked_argmax", "eco_env_results", "eco_graph_aggregate", "eco_mpnn_grad_scratch_bytes", "eco_mpnn_grad", "eco_mpnn_grad_ev", "eco_mpnn_adam", "eco_mpnn_adam_dev", "eco_dp_create", "eco_dp_handle", "eco_dp_open", "eco_dp_adam", "eco_dp_destroy", "eco_mpnn_scratch_bytes", "eco_mpnn_packed_bytes",
+            "eco_env_best_spins", "eco_env_masked_argmax", "eco_env_results", "eco_graph_aggregate", "eco_mpnn_grad_scratch_bytes", "eco_mpnn_grad", "eco_mpnn_grad_ev", "eco_mpnn_adam", "eco_mpnn_adam_dev", "eco_dqn_masked_td_target", "eco_dqn_masked_argmax", "eco_dqn_masked_explore", "eco_mpnn_grad_obs", "eco_dp_create", "eco_dp_handle", "eco_dp_open", "eco_dp_adam", "eco_dp_destroy", "eco_mpnn_scratch_bytes", "eco_mpnn_packed_bytes",
             "eco_mpnn_pack", "eco_mpnn_forward", "eco_rollout", "eco_session_create", "eco_session_destroy",
             "eco_session_rollout", "eco_wgraphs_workspace_bytes", "eco_wgraphs_bind", "eco_wgraphs_load_dev",
             "eco_wenv_workspace_bytes", "eco_wenv_bind", "eco_wenv_reset", "eco_wenv_step", "eco_wmpnn_forward", "eco_wrollout",

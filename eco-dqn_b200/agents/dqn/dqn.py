@@ -13,6 +13,11 @@ gradient clipping), same schedules (dqn.py:467-487), same evaluation metric and 
     gradients are averaged with ONE all-reduce over the flat gradient buffer (NCCL over NVLink), then every rank
     applies the same Adam step.
 
+S2V-DQN (irreversible spins, `observables=[SPIN_STATE]`, `RewardSignal.DENSE`, `MPNN(n_obs_in=1)`; reference dqn.py with
+`reversible_spins=False`) trains on the same kernels: episodes start from all -1, actions, targets and `predict` only choose
+spins still at -1 (csrc/dqn_masked.cu), and the 1-observable network is trained as a zero-padded 7-observable "shadow"
+whose storage the kernels alias (`agent.network` shows its live columns; `save()` writes the 1-observable state_dict).
+
 Differences from the reference that a caller can see: `test_metric` defaults to TestMetric.BEST (the reference's
 default ENERGY_ERROR has no branch left in its evaluate_agent and always scores 0); BEST and FINAL are supported.
 `logging` is accepted and ignored (the reference's pickle Logger is out of scope; every script passes False).
@@ -31,9 +36,29 @@ from ... import engine, sharding
 from ... import _lib
 from ..._lib import lib, check
 from .utils import KernelAdam, ReplayBuffer, TestMetric, set_global_seed
-from ...envs.utils import OptimisationTarget
+from ...envs.utils import OptimisationTarget, Observable, RewardSignal
+from ...networks.mpnn import MPNN
 
 import ctypes as C
+
+
+def padded_shadow(net, device):
+    """The 7-observable MPNN that trains a 1-observable (S2V-DQN) one: it holds `net`'s values with zero columns for the six
+    observables `net` does not see, and `net`'s parameters become views of the shadow's (the live columns of W_init / W_e,
+    the shadow's own tensors elsewhere), so the kernels, Adam and the module read and write the same storage.  Gradients
+    with exactly zero padded columns (eco_mpnn_grad_obs) keep those columns at exactly 0.0 through Adam."""
+    with torch.random.fork_rng(devices=[]):             # building the shadow draws no numbers the reference would not
+        shadow = MPNN(n_obs_in=7).to(device)
+    own = dict(net.named_parameters())
+    for name, sp in shadow.named_parameters():
+        p = own[name]
+        with torch.no_grad():
+            sp.zero_()
+            sp[..., :p.shape[-1]].copy_(p)
+        mod_name, _, leaf = name.rpartition(".")
+        setattr(net.get_submodule(mod_name), leaf, sp if p.shape == sp.shape else torch.nn.Parameter(sp.detach()[:, :p.shape[1]]))
+    net._engine_cache = None
+    return shadow
 
 
 class DQN:
@@ -98,9 +123,9 @@ class DQN:
             envs = [envs]
         self.envs = envs
         self._check_uniform(envs, "training")
-        if any(not e.reversible_spins for e in envs):
-            raise NotImplementedError("irreversible (S2V-DQN) environments are outside the accelerated path")
-        self.acting_in_reversible_spin_env = True
+        self.acting_in_reversible_spin_env = bool(envs[0].reversible_spins)
+        if not self.acting_in_reversible_spin_env:
+            self._check_s2v(envs, "training")
         self.n_spins, self.max_steps = envs[0].n_spins, envs[0].max_steps
         self.basin_reward = envs[0].basin_reward
         self.min_cut = envs[0].optimisation_target == OptimisationTarget.MIN_CUT
@@ -112,6 +137,10 @@ class DQN:
         self._gen.manual_seed(self.seed + 7919 * self.rank)
 
         self.network = network().to(self.device)
+        if not self.acting_in_reversible_spin_env and getattr(self.network, "n_obs_in", None) != 1:
+            raise NotImplementedError("irreversible (S2V-DQN) environments observe the spins only: the network must be "
+                                      "MPNN(n_obs_in=1)")
+        self._qnet = self.network                 # the module whose storage the kernels read and Adam updates in place
         self.init_network_params = init_network_params
         self.init_weight_std = init_weight_std
         if init_network_params is not None:
@@ -121,16 +150,19 @@ class DQN:
                 for m in self.network.modules():
                     if type(m) == torch.nn.Linear:
                         m.weight.normal_(0, init_weight_std)
+        if not self.acting_in_reversible_spin_env:
+            self._qnet = padded_shadow(self.network, self.device)
         if self.world > 1:                       # every rank starts from rank 0's parameters
-            for p in self.network.parameters():
+            for p in self._qnet.parameters():
                 torch.distributed.broadcast(p.data, src=0)
         self.target_network = network().to(self.device)
         self.target_network.load_state_dict(self.network.state_dict())
-        for p in self.target_network.parameters():
+        self._qnet_target = padded_shadow(self.target_network, self.device) if self._qnet is not self.network else self.target_network
+        for p in list(self.target_network.parameters()) + list(self._qnet_target.parameters()):
             p.requires_grad = False
-        if self.network.engine_weights(self.device).aliases:
+        if self._qnet.engine_weights(self.device).aliases:
             # Adam in one hand-written kernel over the live parameters (eco_mpnn_adam)
-            self.optimizer = KernelAdam(self.network, lr=self.initial_learning_rate, eps=self.adam_epsilon,
+            self.optimizer = KernelAdam(self._qnet, lr=self.initial_learning_rate, eps=self.adam_epsilon,
                                         weight_decay=self.weight_decay)
         else:
             self.optimizer = optim.Adam(self.network.parameters(), lr=self.initial_learning_rate, eps=self.adam_epsilon,
@@ -142,15 +174,20 @@ class DQN:
         else:
             self.test_envs = test_envs if type(test_envs) == list else [test_envs]
         self._check_uniform(self.test_envs, "test")
-        if any(not e.reversible_spins for e in self.test_envs):
-            raise NotImplementedError("irreversible (S2V-DQN) environments are outside the accelerated path")
+        if self.test_envs[0].reversible_spins != self.acting_in_reversible_spin_env:
+            raise NotImplementedError("training and test environments must both be ECO-DQN (reversible spins) or both "
+                                      "S2V-DQN (irreversible spins)")
+        if not self.acting_in_reversible_spin_env:
+            self._check_s2v(self.test_envs, "test")
         self.test_episodes = int(test_episodes)
         self.test_frequency = test_frequency
         self.test_save_path = test_save_path
         self.test_metric = test_metric
         self.losses_save_path = os.path.join(os.path.split(self.test_save_path)[0], "losses.pkl")
         self.solution_save_path = os.path.join(os.path.split(self.test_save_path)[0], "solution.pkl")
-        self.allowed_action_state = (-1, 1)
+        self.allowed_action_state = (-1, 1) if self.acting_in_reversible_spin_env else -1
+        # lock-step: every episode ends together -- after max_steps, or, with irreversible spins, once no spin is left at -1
+        self._episode_steps = self.max_steps if self.acting_in_reversible_spin_env else min(self.max_steps, self.n_spins)
         self.save_network_frequency = save_network_frequency
         self.network_save_path = network_save_path
 
@@ -168,7 +205,8 @@ class DQN:
         ring[:] = engine.graphs_to_int8(first[0])[0]          # placeholder so that every slot holds a valid graph
         self._graphs = engine.GraphSet(ring, device=self.device, min_cut=self.min_cut)
         self._ring_pos = 0
-        self._env = engine.BatchedSpinSystem(self._graphs, E, T, self.basin_reward)
+        rev = self.acting_in_reversible_spin_env
+        self._env = engine.BatchedSpinSystem(self._graphs, E, T, self.basin_reward, reversible_spins=rev, dense_reward=not rev)
         self.replay_buffer = ReplayBuffer(replay_buffer_size, self._env.NP, self.device)
         self.replay_buffers = {n: self.replay_buffer}
         self._start_episodes(first)
@@ -200,6 +238,17 @@ class DQN:
                 raise NotImplementedError("all %s environments must share %s (got %s)" %
                                           (what, attr, sorted(set(str(getattr(e, attr)) for e in envs))))
 
+    @staticmethod
+    def _check_s2v(envs, what):
+        """Irreversible spins are trained in the reference's S2V-DQN configuration only (dqn.py with reversible_spins=False,
+        train_eco.py:311-315): spin-state observation, dense reward, no basin reward."""
+        for e in envs:
+            obs = [o for _, o in e.observables]
+            if obs != [Observable.SPIN_STATE] or e.reward_signal != RewardSignal.DENSE or e.basin_reward is not None:
+                raise NotImplementedError("irreversible spins are supported in the S2V-DQN configuration only "
+                                          "(observables=[SPIN_STATE], RewardSignal.DENSE, basin_reward=None); got a %s "
+                                          "environment with %s, %s, basin_reward=%s" % (what, obs, e.reward_signal, e.basin_reward))
+
     def _new_graph(self):
         env = random.sample(self.envs, k=1)[0]                # get_random_env, dqn.py:242-248
         return np.asarray(env.gg.get())
@@ -229,7 +278,10 @@ class DQN:
         if graphs is None:
             graphs = [self._new_graph() for _ in range(E)]
         slots = self._write_ring(graphs)
-        spins = np.stack([2 * np.random.randint(2, size=self.n_spins) - 1 for _ in range(E)])   # spinsystem.py:294
+        if self.acting_in_reversible_spin_env:
+            spins = np.stack([2 * np.random.randint(2, size=self.n_spins) - 1 for _ in range(E)])   # spinsystem.py:294
+        else:
+            spins = -np.ones((E, self.n_spins), dtype=np.int8)       # irreversible spins start at -1 (no draws)
         self._env.reset(spins=spins, graph_idx=slots)
         if getattr(self, "_scores", None) is None:
             self._scores = torch.zeros(E, dtype=torch.float64, device=self.device)
@@ -239,7 +291,10 @@ class DQN:
     def _obs_from(self, xn, xg, graph):
         """[B, 7 + N, N] fp32 observations in the reference's layout, rebuilt on the device for the autograd forward."""
         n = self.n_spins
-        rows = torch.cat([xn[:, :, :n], xg.unsqueeze(-1).expand(-1, -1, n)], dim=1)
+        if getattr(self.network, "n_obs_in", 7) == 1:          # S2V-DQN: [B, 1 + N, N], the spin row only
+            rows = xn[:, :1, :n]
+        else:
+            rows = torch.cat([xn[:, :, :n], xg.unsqueeze(-1).expand(-1, -1, n)], dim=1)
         adj = self._graphs.J[graph.long(), :n, :n].to(torch.float32)
         return torch.cat([rows, adj], dim=1)
 
@@ -256,6 +311,28 @@ class DQN:
                                      engine._ptr(xg), float(norm_max), engine._ptr(q), engine._ptr(act),
                                      engine._ptr(scratch), self._env.mpnn_impl, engine._stream()))
         return (q[:, :self.n_spins] if want_q else None), act
+
+    def _masked_td_target(self, q_online, q_target, t):
+        """S2V-DQN TD target (dqn.py:416-432 with irreversible spins) in one kernel: masked Double-DQN argmax / masked max over
+        the spins of s' still at -1, clip, r + (1 - done) * gamma * q.  q_* as _q_kernel returns them ([B, N] views of
+        [B, NP] rows).  Returns td [B] fp32."""
+        B = q_target.shape[0]
+        td = torch.empty(B, dtype=torch.float32, device=self.device)
+        xn_next = t["xn_next"].contiguous()
+        reward, done = t["reward"].to(torch.float32).contiguous(), t["done"].to(torch.float32).contiguous()
+        check(lib().eco_dqn_masked_td_target(B, self.n_spins, q_target.stride(0),
+                                             engine._ptr(q_online if self.double_dqn else None), engine._ptr(q_target),
+                                             engine._ptr(xn_next), engine._ptr(reward), engine._ptr(done), float(self.gamma),
+                                             int(self.double_dqn), int(bool(self.clip_Q_targets)), engine._ptr(td), None,
+                                             engine._stream()))
+        return td
+
+    def _masked_argmax(self, q, xn):
+        """argmax over the vertices whose row-0 feature is -1 (spins still at -1), per row; q [B, N] view of [B, NP] rows."""
+        act = torch.empty(q.shape[0], dtype=torch.int32, device=self.device)
+        check(lib().eco_dqn_masked_argmax(q.shape[0], self.n_spins, q.stride(0), engine._ptr(q), engine._ptr(xn.contiguous()),
+                                          engine._ptr(act), engine._stream()))
+        return act
 
     # ------------------------------------------------------------------ learning
     def learn(self, timesteps, verbose=False):
@@ -287,7 +364,7 @@ class DQN:
                 self.replay_buffer.add(xn, xg, actions, reward, env.xn, env.xg, done, graph)
             t_before, timestep = timestep, timestep + E
 
-            if env.current_step == self.max_steps:            # lock-step: every episode ends together
+            if env.current_step == self._episode_steps:       # lock-step: every episode ends together
                 if verbose:
                     losses_eps = [float(x) for x in losses_eps]
                     loss_str = "{:.2e}".format(np.mean(losses_eps)) if (is_training_ready and losses_eps) else "N/A"
@@ -305,8 +382,8 @@ class DQN:
                     losses.append([timestep, loss])
                     losses_eps.append(loss)
                 if self._crossings(t_before, timestep, self.update_target_frequency):
-                    self.target_network.load_state_dict(self.network.state_dict())
-                    self.target_network.engine_weights(self.device)      # re-pack now: a replayed graph would not
+                    self._qnet_target.load_state_dict(self._qnet.state_dict())
+                    self._qnet_target.engine_weights(self.device)        # re-pack now: a replayed graph would not
 
             if self._crossings(t_before + 1, timestep + 1, self.test_frequency) and self.evaluate and is_training_ready:
                 test_score, test_solution = self.evaluate_agent()
@@ -357,6 +434,11 @@ class DQN:
             gc = self._graphs_nm                       # norm_max = 0 -> the kernels read *dmax = _nm_buf
 
             def td_target_of():
+                if not self.acting_in_reversible_spin_env:
+                    q_on = self._q_kernel(self._qnet, t["xn_next"], t["xg_next"], graph, 0.0, graphs_c=gc)[0] \
+                        if self.double_dqn else None
+                    q_tgt, _ = self._q_kernel(self._qnet_target, t["xn_next"], t["xg_next"], graph, 0.0, graphs_c=gc)
+                    return self._masked_td_target(q_on, q_tgt, t)
                 if self.double_dqn:
                     _, greedy = self._q_kernel(self.network, t["xn_next"], t["xg_next"], graph, 0.0, want_q=False, graphs_c=gc)
                     q_tgt, _ = self._q_kernel(self.target_network, t["xn_next"], t["xg_next"], graph, 0.0, graphs_c=gc)
@@ -388,7 +470,7 @@ class DQN:
             if self.world > 1 and not self._fused_dp:
                 self._allreduce_grads()
             if self.max_grad_norm is not None:
-                torch.nn.utils.clip_grad_norm_(self.network.parameters(), self.max_grad_norm)
+                torch.nn.utils.clip_grad_norm_(self._qnet.parameters(), self.max_grad_norm)
             self.optimizer.step()
         return loss
 
@@ -398,27 +480,36 @@ class DQN:
         graph = t["graph"]
         with torch.no_grad():
             norm_max = float(self._graphs.gstat[graph.long(), 0].max().clamp(min=1).item())
-            if self.double_dqn:
+            if not self.acting_in_reversible_spin_env:
+                q_on = self._q_kernel(self._qnet, t["xn_next"], t["xg_next"], graph, norm_max)[0] if self.double_dqn else None
+                q_tgt, _ = self._q_kernel(self._qnet_target, t["xn_next"], t["xg_next"], graph, norm_max)
+                td_target = self._masked_td_target(q_on, q_tgt, t).unsqueeze(1)
+            elif self.double_dqn:
                 _, greedy = self._q_kernel(self.network, t["xn_next"], t["xg_next"], graph, norm_max, want_q=False)
                 q_tgt, _ = self._q_kernel(self.target_network, t["xn_next"], t["xg_next"], graph, norm_max)
                 q_value_target = q_tgt.gather(1, greedy.long().unsqueeze(1))
             else:
                 q_tgt, _ = self._q_kernel(self.target_network, t["xn_next"], t["xg_next"], graph, norm_max)
                 q_value_target = q_tgt.max(1, True)[0]
-            if self.clip_Q_targets:
-                q_value_target[q_value_target < 0] = 0
-            td_target = t["reward"].unsqueeze(1) + (1 - t["done"].unsqueeze(1)) * self.gamma * q_value_target
+            if self.acting_in_reversible_spin_env:
+                if self.clip_Q_targets:
+                    q_value_target[q_value_target < 0] = 0
+                td_target = t["reward"].unsqueeze(1) + (1 - t["done"].unsqueeze(1)) * self.gamma * q_value_target
         q_all = self.network(self._obs_from(t["xn"], t["xg"], graph))
         if q_all.dim() == 1:
             q_all = q_all.unsqueeze(0)
         q_value = q_all.gather(1, t["action"].unsqueeze(1))
         loss = self.loss(q_value, td_target, reduction='mean')
         self.optimizer.zero_grad()
+        if self._qnet is not self.network:
+            self.network.zero_grad(set_to_none=True)
         loss.backward()
         if self.world > 1:
             sharding.allreduce_mean_grads(self.network.parameters())
+        if self._qnet is not self.network:
+            self._pad_grads()
         if self.max_grad_norm is not None:
-            torch.nn.utils.clip_grad_norm_(self.network.parameters(), self.max_grad_norm)
+            torch.nn.utils.clip_grad_norm_(self._qnet.parameters(), self.max_grad_norm)
         if isinstance(self.optimizer, KernelAdam):
             scale, self.optimizer.grad_scale = self.optimizer.grad_scale, 1.0      # (already averaged)
             dp, self.optimizer._dp = self.optimizer._dp, None
@@ -427,6 +518,17 @@ class DQN:
         else:
             self.optimizer.step()
         return loss.detach()
+
+    def _pad_grads(self):
+        """Autograd gradients of the 1-observable module -> the shadow's parameters (zero in the padded columns)."""
+        own = dict(self.network.named_parameters())
+        for name, sp in self._qnet.named_parameters():
+            p = own[name]
+            if p is sp or p.grad is None:
+                continue
+            g = torch.zeros_like(sp)
+            g[:, :p.shape[1]] = p.grad
+            sp.grad = g
 
     def _train_step_device(self, idx):
         """The update for the replay rows `idx` (device int64 [minibatch]); with cuda_graph the captured update is replayed."""
@@ -444,7 +546,7 @@ class DQN:
         NCCL channels) are real updates, so parameters and optimizer state are saved before and put back after."""
         opt = self.optimizer
         self._g_idx = idx.clone()
-        saved = [p.detach().clone() for p in self.network.parameters()]
+        saved = [p.detach().clone() for p in self._qnet.parameters()]
         state = (opt.exp_avg.clone(), opt.exp_avg_sq.clone(), opt.step_dev.clone())
         opt.sync_lr()
         side = torch.cuda.Stream(device=self.device)
@@ -457,10 +559,10 @@ class DQN:
 
         def restore():
             with torch.no_grad():
-                for p, q in zip(self.network.parameters(), saved):
+                for p, q in zip(self._qnet.parameters(), saved):
                     p.copy_(q)
                 opt.exp_avg.copy_(state[0]); opt.exp_avg_sq.copy_(state[1]); opt.step_dev.copy_(state[2])
-            self.network.engine_weights(self.device).repack()
+            self._qnet.engine_weights(self.device).repack()
         restore()
         if self.world > 1:
             torch.distributed.barrier()       # (the exchange epochs of eco_dp_adam count on their own: nothing to rewind)
@@ -473,7 +575,7 @@ class DQN:
         """loss and d loss / d weights of the regression step (dqn.py:436-447) through eco_mpnn_grad; the gradient
         lands in `p.grad` of every parameter (views of one flat buffer, state_dict order)."""
         B = xn.shape[0]
-        w = self.network.engine_weights(self.device)
+        w = self._qnet.engine_weights(self.device)
         nb = lib().eco_mpnn_grad_scratch_bytes(B, self.n_spins)
         if self._grad_scratch is None or self._grad_scratch.numel() < nb:
             self._grad_scratch = torch.empty(nb, dtype=torch.uint8, device=self.device)
@@ -482,11 +584,20 @@ class DQN:
         xn, xg, graph = xn.contiguous(), xg.contiguous(), graph.to(torch.int32).contiguous()
         action = action.to(torch.int32).contiguous()
         target = td_target.reshape(-1).to(torch.float32).contiguous()
-        check(lib().eco_mpnn_grad_ev(C.byref(self._graphs.c if graphs_c is None else graphs_c), C.byref(w.c), B, engine._ptr(graph),
-                                     engine._ptr(xn), engine._ptr(xg), float(norm_max), engine._ptr(action), engine._ptr(target),
-                                     self._loss_kind, engine._ptr(loss), engine._ptr(flat), engine._ptr(self._grad_scratch),
-                                     C.c_void_p(ready.cuda_event if ready is not None else 0), engine._stream()))
-        params = dict(self.network.named_parameters())
+        gcs = C.byref(self._graphs.c if graphs_c is None else graphs_c)
+        ev = C.c_void_p(ready.cuda_event if ready is not None else 0)
+        if self._qnet is self.network:
+            check(lib().eco_mpnn_grad_ev(gcs, C.byref(w.c), B, engine._ptr(graph),
+                                         engine._ptr(xn), engine._ptr(xg), float(norm_max), engine._ptr(action), engine._ptr(target),
+                                         self._loss_kind, engine._ptr(loss), engine._ptr(flat), engine._ptr(self._grad_scratch),
+                                         ev, engine._stream()))
+        else:
+            # the 1-observable network trained as its 7-observable shadow: the padded columns' gradient is exactly zero
+            check(lib().eco_mpnn_grad_obs(gcs, C.byref(w.c), B, engine._ptr(graph), engine._ptr(xn), engine._ptr(xg),
+                                          float(norm_max), engine._ptr(action), engine._ptr(target), self._loss_kind, 1,
+                                          engine._ptr(loss), engine._ptr(flat), engine._ptr(self._grad_scratch), ev,
+                                          engine._stream()))
+        params = dict(self._qnet.named_parameters())
         off = 0
         for key, shp in zip(engine.STATE_DICT_KEYS, engine.STATE_DICT_SHAPES):
             n = int(np.prod(shp))
@@ -496,6 +607,10 @@ class DQN:
                 g = g[:, :p.shape[1]].contiguous()
             p.grad = g
             off += n
+        if self._qnet is not self.network:       # the module's own W_init / W_e see the live columns of the gradient
+            for key, p in self.network.named_parameters():
+                if p is not params[key]:
+                    p.grad = params[key].grad[:, :p.shape[1]]
         return loss
 
     def _allreduce_grads(self):
@@ -531,10 +646,13 @@ class DQN:
     def _act_body(self):
         rb, env, E, dev = self.replay_buffer, self._env, self.n_envs, self.device
         self._ag_xn.copy_(env.xn); self._ag_xg.copy_(env.xg); self._ag_graph.copy_(env.graph_idx)
-        rand_actions = torch.randint(0, self.n_spins, (E,), device=dev, generator=self._gen, dtype=torch.int32)
-        greedy = self._q_kernel(self.network, self._ag_xn, self._ag_xg, self._ag_graph, -1.0, want_q=False)[1]
-        explore = torch.rand(E, device=dev, generator=self._gen) < self._ag_eps
-        actions = torch.where(self._ag_ready & ~explore, greedy, rand_actions).contiguous()
+        if self.acting_in_reversible_spin_env:
+            rand_actions = torch.randint(0, self.n_spins, (E,), device=dev, generator=self._gen, dtype=torch.int32)
+            greedy = self._q_kernel(self.network, self._ag_xn, self._ag_xg, self._ag_graph, -1.0, want_q=False)[1]
+            explore = torch.rand(E, device=dev, generator=self._gen) < self._ag_eps
+            actions = torch.where(self._ag_ready & ~explore, greedy, rand_actions).contiguous()
+        else:
+            actions = self._masked_explore(self._ag_xn, self._ag_xg, self._ag_graph, self._ag_eps, self._ag_ready)
         with torch.cuda.device(dev):
             check(lib().eco_env_step(C.byref(env.gs.c), C.byref(env.c), _lib.POLICY_ACTIONS, engine._ptr(actions),
                                      engine._ptr(env._reward), engine._ptr(env._done), None, None, None, engine._stream()))
@@ -574,16 +692,38 @@ class DQN:
         with torch.cuda.graph(self._ag):
             self._act_body()
 
+    def _masked_explore(self, xn, xg, graph, eps_dev, ready_dev):
+        """Irreversible spins, several lock-step environments: the epsilon-greedy action of every environment of the trainer's
+        batch among its spins still at -1 (eco_dqn_masked_explore; two device uniforms per environment from the agent's
+        generator, epsilon and the "training ready" flag read from device memory, so the step can be captured)."""
+        E = xn.shape[0]
+        u = torch.rand(E, 2, device=self.device, generator=self._gen)
+        q = self._q_kernel(self._qnet, xn, xg, graph, -1.0)[0]
+        actions = torch.empty(E, dtype=torch.int32, device=self.device)
+        check(lib().eco_dqn_masked_explore(C.byref(self._env.c), engine._ptr(q), engine._ptr(u), engine._ptr(eps_dev),
+                                           engine._ptr(ready_dev), engine._ptr(actions), engine._stream()))
+        return actions
+
     def act(self, state, is_training_ready=True):
         """epsilon-greedy (reference dqn.py:453-465).  One environment: the reference's own draws, in its order
-        (`random.uniform(0, 1) >= epsilon` -> greedy, else `np.random.randint(0, n)`), so a seeded run picks the
-        reference's actions.  Several lock-step environments: one device draw per environment."""
+        (`random.uniform(0, 1) >= epsilon` -> greedy, else `np.random.randint(0, n)`, with irreversible spins one
+        `np.random.randint(0, k)` over the k spins still at -1 in ascending order), so a seeded run picks the reference's
+        actions.  Several lock-step environments: one device draw per environment (irreversible spins: the state is that
+        of the trainer's own environments, see _masked_explore)."""
         xn, xg, graph = state
         E = xn.shape[0]
         if E == 1:
             if is_training_ready and random.uniform(0, 1) >= self.epsilon:
                 return self.predict(state)
-            return torch.tensor([np.random.randint(0, self.n_spins)], dtype=torch.int32, device=self.device)
+            if self.acting_in_reversible_spin_env:
+                return torch.tensor([np.random.randint(0, self.n_spins)], dtype=torch.int32, device=self.device)
+            allowed = np.flatnonzero(xn[0, 0, :self.n_spins].cpu().numpy() == self.allowed_action_state)
+            a = int(allowed[np.random.randint(0, len(allowed))]) if len(allowed) else 0
+            return torch.tensor([a], dtype=torch.int32, device=self.device)
+        if not self.acting_in_reversible_spin_env:
+            eps = torch.full((1,), float(self.epsilon), dtype=torch.float32, device=self.device)
+            ready = torch.full((1,), bool(is_training_ready), dtype=torch.bool, device=self.device)
+            return self._masked_explore(xn, xg, graph, eps, ready)
         rand_actions = torch.randint(0, self.n_spins, (E,), device=self.device, generator=self._gen, dtype=torch.int32)
         if not is_training_ready:
             return rand_actions
@@ -594,9 +734,13 @@ class DQN:
     @torch.no_grad()
     def predict(self, states, acting_in_reversible_spin_env=None):
         """argmax_a Q(s, a) per environment; every environment is normalised by its own graph, like the reference's
-        one-environment forward (dqn.py:490-503)."""
+        one-environment forward (dqn.py:490-503).  Irreversible spins: argmax over the spins still at -1 (dqn.py:504-512)."""
         xn, xg, graph = states
-        return self._q_kernel(self.network, xn, xg, graph, -1.0, want_q=False)[1]
+        rev = self.acting_in_reversible_spin_env if acting_in_reversible_spin_env is None else acting_in_reversible_spin_env
+        if rev:
+            return self._q_kernel(self._qnet, xn, xg, graph, -1.0, want_q=False)[1]
+        q = self._q_kernel(self._qnet, xn, xg, graph, -1.0)[0]
+        return self._masked_argmax(q, xn)
 
     def update_epsilon(self, timestep):
         eps = self.initial_exploration_rate - (self.initial_exploration_rate - self.final_exploration_rate) * (
@@ -624,24 +768,28 @@ class DQN:
         The reference fills `batch_size` (default: the minibatch size) slots, steps them together -- so `norm.max()`
         (mpnn.py:102) is the largest degree among the graphs of that group -- and refills when the group is done; per
         episode it draws, in order, the environment (`random.sample`), the graph (`gg.get()`) and the spins
-        (`np.random.randint`).  Same draws, same groups here; every group is one device rollout."""
+        (`np.random.randint`).  Same draws, same groups here; every group is one device rollout.  Irreversible spins
+        (S2V-DQN): every episode starts from all -1 (no spin draws) and the rollout takes the masked argmax."""
         k = self.test_episodes
         bsz = self.minibatch_size if batch_size is None else int(batch_size)
         graphs, spins = [], []
         for _ in range(k):
             e = random.sample(self.test_envs, k=1)[0]                        # get_random_env, dqn.py:242-248
             graphs.append(np.asarray(e.gg.get()))                            # env.reset(): spinsystem.py:188-198
-            spins.append(2 * np.random.randint(2, size=self.n_spins) - 1)    # spinsystem.py:294
+            if self.acting_in_reversible_spin_env:
+                spins.append(2 * np.random.randint(2, size=self.n_spins) - 1)    # spinsystem.py:294
         t_env = self.test_envs[0]
+        rev = self.acting_in_reversible_spin_env
         gs = engine.GraphSet(np.stack(graphs), device=self.device,
                              min_cut=t_env.optimisation_target == OptimisationTarget.MIN_CUT)
         deg = gs.gstat[:, 0].cpu().numpy()
-        w = self.network.engine_weights(self.device)
+        w = self._qnet.engine_weights(self.device)
         scores, sols = np.zeros(k), np.zeros(k)
         for g0 in range(0, k, bsz):
             g1 = min(k, g0 + bsz)
-            env = engine.BatchedSpinSystem(gs, g1 - g0, t_env.max_steps, t_env.basin_reward)
-            env.reset(spins=np.stack(spins[g0:g1]), graph_idx=np.arange(g0, g1, dtype=np.int32))
+            env = engine.BatchedSpinSystem(gs, g1 - g0, t_env.max_steps, t_env.basin_reward, reversible_spins=rev,
+                                           dense_reward=not rev)
+            env.reset(spins=np.stack(spins[g0:g1]) if rev else None, graph_idx=np.arange(g0, g1, dtype=np.int32))
             env.rollout(w, norm_max=float(max(1, deg[g0:g1].max())))
             ep = env.episodes()
             if self.test_metric == TestMetric.BEST:
@@ -654,7 +802,11 @@ class DQN:
     def save(self, path='network.pth'):
         if os.path.dirname(path):
             os.makedirs(os.path.dirname(path), exist_ok=True)
-        torch.save(self.network.state_dict(), path)
+        if self._qnet is self.network:
+            torch.save(self.network.state_dict(), path)
+        else:   # the module's W_init / W_e are views into the shadow: save their own [64, 1] / [63, 2] data only
+            torch.save({k: v.detach().clone(memory_format=torch.contiguous_format)
+                        for k, v in self.network.state_dict().items()}, path)
 
     def load(self, path):
-        self.network.load_state_dict(torch.load(path, map_location=self.device))
+        self.network.load_state_dict(torch.load(path, map_location=self.device))   # (S2V-DQN: writes through to the shadow)

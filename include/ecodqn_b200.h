@@ -267,6 +267,41 @@ int    eco_mpnn_adam_dev(const eco_mpnn_t* w, const float* grad_dev, float* exp_
                          int32_t* step_dev, const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
                          float grad_scale, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * S2V-DQN training (irreversible spins, reference src/agents/dqn/dqn.py with reversible_spins=False): the agent may only
+ * flip a spin still at -1.  Masking rule of eco_env_masked_argmax throughout: a disallowed entry compares as -1000.0, the
+ * lowest index wins ties, a row with no allowed vertex picks action 0.
+ *
+ * eco_dqn_masked_td_target (dqn.py:416-432): td_dev[b] = reward[b] + (1 - done[b]) * gamma * q, where q is
+ *   double_dqn: q_target[b, argmax_masked q_online[b, :]]   else: max_masked q_target[b, :]
+ * then clipped at 0 when `clip`.  An action is allowed where row 0 of the next-state features is -1.0.  q_* [B, NP] fp32
+ * (as eco_mpnn_forward writes them), xn_next_dev [B, 3, NP], reward_dev / done_dev [B] fp32; q_online_dev may be NULL
+ * when double_dqn == 0.  chosen_dev [B] int32 (optional) receives the index q was taken at.  Bit-identical to the torch
+ * expression of the reference evaluated in fp32 (no FMA contraction).
+ *
+ * eco_dqn_masked_argmax (dqn.py:504-512): actions_dev[b] = argmax over the allowed vertices of q_dev[b, :], the mask from
+ * row 0 of xn_dev [B, 3, NP].
+ *
+ * eco_dqn_masked_explore (dqn.py:453-465): epsilon-greedy action of every environment of `env`: the masked argmax of
+ * q_dev [B, NP] when *ready_dev != 0 and uniforms_dev[2b] >= *eps_dev, otherwise the k-th spin still at -1 in ascending
+ * vertex order, k = min(floor(uniforms_dev[2b + 1] * c), c - 1) with c the number of such spins.  No host read: capturable.
+ *
+ * eco_mpnn_grad_obs: eco_mpnn_grad_ev for a network with n_obs_in observables (1 = S2V-DQN, 7 = ECO-DQN).  The weights
+ * `w` points at are the 7-observable layout; for n_obs_in = 1 the gradient of the zero-padded columns (W_init[:, 1:7],
+ * W_e[:, 2:8]) is written as exactly 0.0, so an Adam step keeps those columns at exactly 0.0.
+ * --------------------------------------------------------------------------------------------------------- */
+int eco_dqn_masked_td_target(int32_t B, int32_t N, int32_t NP, const float* q_online_dev, const float* q_target_dev,
+                             const float* xn_next_dev, const float* reward_dev, const float* done_dev, float gamma,
+                             int32_t double_dqn, int32_t clip, float* td_dev, int32_t* chosen_dev, void* stream);
+int eco_dqn_masked_argmax(int32_t B, int32_t N, int32_t NP, const float* q_dev, const float* xn_dev, int32_t* actions_dev,
+                          void* stream);
+int eco_dqn_masked_explore(const eco_env_t* env, const float* q_dev, const float* uniforms_dev, const float* eps_dev,
+                           const uint8_t* ready_dev, int32_t* actions_dev, void* stream);
+int eco_mpnn_grad_obs(const eco_graphs_t* g, const eco_mpnn_t* w, int32_t B, const int32_t* graph_idx_dev,
+                      const float* xn_dev, const float* xg_dev, float norm_max, const int32_t* actions_dev,
+                      const float* targets_dev, int32_t loss_kind, int32_t n_obs_in, float* loss_dev, float* grad_dev,
+                      void* scratch_dev, void* targets_ready_event, void* stream);
+
 /* Data-parallel form of the update (SURVEY.md section 8e; the reference is single-process: src/agents/dqn/dqn.py:403-451
  * runs on one device).  One process per GPU of one NVSwitch box; every rank calls eco_dp_adam once per update with ITS
  * gradient and gets the Adam step of the MEAN gradient applied to its parameters: the kernel publishes the gradient in a
