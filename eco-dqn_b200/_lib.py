@@ -150,6 +150,8 @@ def lib():
         "eco_smpnn_scratch_bytes": (C.c_size_t, [i32, i32]),
         "eco_smpnn_forward": (C.c_int, [P(SGraphs), P(Mpnn), i32, vp, vp, vp, C.c_float, vp, vp, vp, vp]),
         "eco_srollout": (C.c_int, [P(SGraphs), P(Env), P(Mpnn), i32, i32, C.c_float, vp, vp, vp, vp, vp, vp]),
+        "eco_smpnn_forward_impl": (C.c_int, [P(SGraphs), P(Mpnn), i32, vp, vp, vp, C.c_float, vp, vp, vp, i32, vp]),
+        "eco_srollout_impl": (C.c_int, [P(SGraphs), P(Env), P(Mpnn), i32, i32, C.c_float, vp, vp, i32, vp, vp, vp, vp]),
         "eco_session_create": (C.c_int, [P(vp), i32, i32, i32, i32, C.c_double, P(vp), i32]),
         "eco_session_destroy": (None, [vp]),
         "eco_session_rollout": (C.c_int, [vp, vp, vp, vp, i32, C.c_float, vp, vp, vp]),
@@ -171,7 +173,7 @@ EXPORTED = ["eco_last_error", "eco_abi_version", "eco_launch_count", "eco_profil
             "eco_wenv_workspace_bytes", "eco_wenv_bind", "eco_wenv_reset", "eco_wenv_step", "eco_wmpnn_forward", "eco_wrollout",
             "eco_wenv_results", "eco_sgraphs_workspace_bytes", "eco_sgraphs_bind", "eco_sgraphs_load_dev",
             "eco_senv_workspace_bytes", "eco_senv_bind", "eco_senv_reset", "eco_senv_step", "eco_smpnn_scratch_bytes",
-            "eco_smpnn_forward", "eco_srollout"]
+            "eco_smpnn_forward", "eco_srollout", "eco_smpnn_forward_impl", "eco_srollout_impl"]
 
 
 def check(rc):

@@ -716,13 +716,42 @@ int eco_smpnn_forward(const eco_sgraphs_t* g, const eco_mpnn_t* w, int32_t B, co
     return launch_smpnn(g, w, B, gidx, xn, xg, norm_max, q, actions, scratch, (cudaStream_t)stream);
 }
 
-int eco_srollout(const eco_sgraphs_t* g, eco_env_t* env, const eco_mpnn_t* w, int32_t n_steps, int32_t policy, float norm_max,
-                 int32_t* act, void* scratch, int32_t* ha, double* hr, double* hs, void* stream) {
+// impl of the CSR-set forward: AUTO / SIMT -> the gather forward with fp32 linears, TCGEN05 -> its linears on the tensor
+// cores (needs eco_mpnn_pack output and a 32-byte aligned scratch: the linears store whole 32-byte sectors)
+static int check_simpl(const eco_mpnn_t* w, int32_t impl, const void* scratch, const char* who) {
+    ECO_CHECK_ARG(impl == ECO_MPNN_AUTO || impl == ECO_MPNN_SIMT || impl == ECO_MPNN_TCGEN05, ECO_ERR_INVALID,
+                  "%s: unknown impl %d", who, impl);
+    if (impl != ECO_MPNN_TCGEN05) return ECO_OK;
+    ECO_CHECK_ARG(w && w->packed, ECO_ERR_INVALID, "%s: the tcgen05 path needs eco_mpnn_pack() output", who);
+    ECO_CHECK_ARG(((uintptr_t)scratch & 31) == 0, ECO_ERR_INVALID, "%s: the tcgen05 path needs a 32-byte aligned scratch", who);
+    return ECO_OK;
+}
+
+int eco_smpnn_forward_impl(const eco_sgraphs_t* g, const eco_mpnn_t* w, int32_t B, const int32_t* gidx, const float* xn,
+                           const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, int32_t impl,
+                           void* stream) {
+    ECO_CHECK_ARG(g && gidx && xn && xg && scratch, ECO_ERR_INVALID, "eco_smpnn_forward_impl: null argument");
+    ECO_CHECK_ARG(B >= 1, ECO_ERR_INVALID, "eco_smpnn_forward_impl: B must be >= 1");
+    ECO_CHECK_ARG(((uintptr_t)scratch & 15) == 0, ECO_ERR_INVALID, "eco_smpnn_forward_impl: scratch must be 16-byte aligned");
+    int rc = check_weights(w, "eco_smpnn_forward_impl");
+    if (rc) return rc;
+    rc = check_simpl(w, impl, scratch, "eco_smpnn_forward_impl");
+    if (rc) return rc;
+    if (impl == ECO_MPNN_TCGEN05)
+        return launch_smpnn_tc(g, w, B, gidx, xn, xg, norm_max, q, actions, scratch, (cudaStream_t)stream);
+    return launch_smpnn(g, w, B, gidx, xn, xg, norm_max, q, actions, scratch, (cudaStream_t)stream);
+}
+
+int eco_srollout_impl(const eco_sgraphs_t* g, eco_env_t* env, const eco_mpnn_t* w, int32_t n_steps, int32_t policy,
+                      float norm_max, int32_t* act, void* scratch, int32_t impl, int32_t* ha, double* hr, double* hs,
+                      void* stream) {
     int rc = check_spair(g, env, "eco_srollout");
     if (rc) return rc;
     ECO_CHECK_ARG(n_steps >= 0, ECO_ERR_INVALID, "eco_srollout: n_steps < 0");
     ECO_CHECK_ARG(policy == ECO_POLICY_NETWORK || policy == ECO_POLICY_GREEDY, ECO_ERR_INVALID,
                   "eco_srollout: policy must be ECO_POLICY_NETWORK or ECO_POLICY_GREEDY");
+    ECO_CHECK_ARG(impl == ECO_MPNN_AUTO || impl == ECO_MPNN_SIMT || impl == ECO_MPNN_TCGEN05, ECO_ERR_INVALID,
+                  "eco_srollout: unknown impl %d", impl);      // (before any launch, the greedy policy's too)
     cudaStream_t st = (cudaStream_t)stream;
     if (policy == ECO_POLICY_GREEDY) {
         for (int t = 0; t < n_steps; ++t) {
@@ -732,13 +761,21 @@ int eco_srollout(const eco_sgraphs_t* g, eco_env_t* env, const eco_mpnn_t* w, in
         return ECO_OK;
     }
     ECO_CHECK_ARG(act && scratch, ECO_ERR_INVALID, "eco_srollout: network policy needs actions and mpnn scratch buffers");
+    rc = check_simpl(w, impl, scratch, "eco_srollout");
+    if (rc) return rc;
     for (int t = 0; t < n_steps; ++t) {
-        rc = eco_smpnn_forward(g, w, env->B, env->graph_idx, env->xn, env->xg, norm_max, nullptr, act, scratch, stream);
+        rc = eco_smpnn_forward_impl(g, w, env->B, env->graph_idx, env->xn, env->xg, norm_max, nullptr, act, scratch, impl,
+                                    stream);
         if (rc) return rc;
         rc = launch_senv_step(g, env, ECO_POLICY_ACTIONS, act, nullptr, nullptr, ha, hr, hs, st);
         if (rc) return rc;
     }
     return ECO_OK;
+}
+
+int eco_srollout(const eco_sgraphs_t* g, eco_env_t* env, const eco_mpnn_t* w, int32_t n_steps, int32_t policy, float norm_max,
+                 int32_t* act, void* scratch, int32_t* ha, double* hr, double* hs, void* stream) {
+    return eco_srollout_impl(g, env, w, n_steps, policy, norm_max, act, scratch, ECO_MPNN_AUTO, ha, hr, hs, stream);
 }
 
 // ------------------------------------------------------------------------------------------------ session

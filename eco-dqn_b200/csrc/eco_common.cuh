@@ -139,6 +139,10 @@ int launch_senv_step(const eco_sgraphs_t* g, eco_env_t* env, int policy, const i
 size_t smpnn_scratch_bytes(int B, int N);
 int launch_smpnn(const eco_sgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn, const float* xg,
                  float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);
+int launch_smpnn_tc(const eco_sgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn, const float* xg,
+                    float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);
+int launch_sparse_linear_tc(const float* A1, const float* A2, int K, long long V, const void* w_packed, float* C,
+                            cudaStream_t st);
 int launch_mpnn_tc(const eco_graphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
                    const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st);
 bool mpnn_tc_can_fuse(const eco_graphs_t* g, const eco_env_t* env);

@@ -8,6 +8,7 @@
 //   src/envs/spinsystem.py:355-559   step                                -> senv_step_kernel
 //   src/agents/solver.py:105-131     Greedy.step                         -> ECO_POLICY_GREEDY inside senv_step_kernel
 //   src/networks/mpnn.py:40-159      MPNN.forward                        -> k_sinit, k_sgather, k_gemm, k_sreadout
+//                                                                          (linears on the tensor cores: sparse_tc.cu)
 //
 // The environment keeps the int8 path's state (eco_env_t: int16 fields, uint16 last-flip steps, the best-diff bitmask, the
 // 96-byte episode block) and its integer / fp64 rules, so for N <= ECO_MAX_SPINS every array equals the dense path's bit for
@@ -27,6 +28,7 @@
 #include "eco_common.cuh"
 #include "env_step_device.cuh"
 #include "mpnn_gemm.cuh"
+#include "mpnn_pack.cuh"
 
 namespace eco {
 
@@ -490,40 +492,63 @@ int launch_senv_step(const eco_sgraphs_t* g, eco_env_t* env, int policy, const i
     return ECO_OK;
 }
 
-// Planes: H ping / pong, E, and two planes that hold P then the aggregate (X) and G then the message (Y).
-int launch_smpnn(const eco_sgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn, const float* xg,
-                 float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st) {
+// Planes: H ping / pong, E, and two planes that hold P then the aggregate (X) and G then the message (Y).  The seven
+// per-vertex linears run as k_gemm (fp32 CUDA cores) or, with `tc`, as sparse_linear_tc_kernel (sparse_tc.cu, tensor
+// cores, bf16 hi/lo operands from eco_mpnn_pack); every other launch is the same.
+static int smpnn_sequence(const eco_sgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn,
+                          const float* xg, float norm_max, float* q, int32_t* actions, void* scratch, bool tc, cudaStream_t st) {
     const int N = g->N, NP = g->NP;
     const long long V = (long long)B * NP;
     const size_t pl = (size_t)V * F;
     float* base = (float*)scratch;
     float *Ha = base, *Hb = base + pl, *E = base + 2 * pl, *X = base + 3 * pl, *Y = base + 4 * pl;
     static unsigned long long attr = 0;
-    if (first_use_on_device(&attr))
+    if (!tc && first_use_on_device(&attr))
         ECO_CUDA(cudaFuncSetAttribute(k_gemm<false, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_smem_bytes(128)));
     const unsigned eblocks = (unsigned)((pl + 255) / 256);
     const unsigned vt = (unsigned)((V + GT - 1) / GT);
+    const uint32_t* pk = static_cast<const uint32_t*>(w->packed);
     prof_begin(ECO_PROF_MPNN, st);
     k_sinit<<<eblocks, 256, 0, st>>>(N, NP, *w, V, xn, xg, Ha, X);
     ECO_LAUNCH_CHECK();
     k_sgather<true><<<eblocks, 256, 0, st>>>(*g, gidx, *w, V, X, Y, norm_max);
     ECO_LAUNCH_CHECK();
-    k_gemm<false, 64><<<vt, 256, gemm_smem_bytes(64), st>>>(Y, nullptr, nullptr, (int)V, w->w_edge_feat, 64, 0, E, 1, 0);
-    ECO_LAUNCH_CHECK();
+    int rc;
+    if (tc) {
+        if ((rc = launch_sparse_linear_tc(Y, nullptr, 64, V, pk + PK_WEF, E, st))) return rc;
+    } else {
+        k_gemm<false, 64><<<vt, 256, gemm_smem_bytes(64), st>>>(Y, nullptr, nullptr, (int)V, w->w_edge_feat, 64, 0, E, 1, 0);
+        ECO_LAUNCH_CHECK();
+    }
     float *Hc = Ha, *Hn = Hb;
     for (int l = 0; l < 3; ++l) {
         k_sgather<false><<<eblocks, 256, 0, st>>>(*g, gidx, *w, V, Hc, X, norm_max);
         ECO_LAUNCH_CHECK();
-        k_gemm<false, 128><<<vt, 256, gemm_smem_bytes(128), st>>>(X, E, nullptr, (int)V, w->w_msg[l], 128, 0, Y, 1, 0);
-        ECO_LAUNCH_CHECK();
-        k_gemm<false, 128><<<vt, 256, gemm_smem_bytes(128), st>>>(Hc, Y, nullptr, (int)V, w->w_upd[l], 128, 0, Hn, 1, 0);
-        ECO_LAUNCH_CHECK();
+        if (tc) {
+            if ((rc = launch_sparse_linear_tc(X, E, 128, V, pk + PK_WM + l * 128 * 64, Y, st))) return rc;
+            if ((rc = launch_sparse_linear_tc(Hc, Y, 128, V, pk + PK_WU + l * 128 * 64, Hn, st))) return rc;
+        } else {
+            k_gemm<false, 128><<<vt, 256, gemm_smem_bytes(128), st>>>(X, E, nullptr, (int)V, w->w_msg[l], 128, 0, Y, 1, 0);
+            ECO_LAUNCH_CHECK();
+            k_gemm<false, 128><<<vt, 256, gemm_smem_bytes(128), st>>>(Hc, Y, nullptr, (int)V, w->w_upd[l], 128, 0, Hn, 1, 0);
+            ECO_LAUNCH_CHECK();
+        }
         float* t = Hc; Hc = Hn; Hn = t;
     }
     k_sreadout<<<(unsigned)B, 256, 0, st>>>(N, NP, *w, Hc, q, actions);
     prof_end(ECO_PROF_MPNN, st);
     ECO_LAUNCH_CHECK();
     return ECO_OK;
+}
+
+int launch_smpnn(const eco_sgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn, const float* xg,
+                 float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st) {
+    return smpnn_sequence(g, w, B, gidx, xn, xg, norm_max, q, actions, scratch, false, st);
+}
+
+int launch_smpnn_tc(const eco_sgraphs_t* g, const eco_mpnn_t* w, int B, const int32_t* gidx, const float* xn, const float* xg,
+                    float norm_max, float* q, int32_t* actions, void* scratch, cudaStream_t st) {
+    return smpnn_sequence(g, w, B, gidx, xn, xg, norm_max, q, actions, scratch, true, st);
 }
 
 }  // namespace eco

@@ -623,19 +623,30 @@ class BatchedSpinSystem:
             self._scratch = torch.empty(nb, dtype=torch.uint8, device=self.device)
         return self._scratch
 
+    def _sparse_impl(self, weights, impl):
+        """The Q-network of a CSR set: AUTO / SIMT run the gather forward with fp32 linears (eco_smpnn_forward), TCGEN05
+        its per-vertex linears on the tensor cores (eco_smpnn_forward_impl), which read the packed bf16 hi/lo weights."""
+        use = self.mpnn_impl if impl is None else impl
+        if use == _lib.MPNN_TCGEN05 and weights is not None and weights._packed is None:
+            raise ValueError("the tensor-core Q-network needs packed weights: MPNNWeights(..., pack=True)")
+        return use
+
     def q_values(self, weights, norm_max=None, want_actions=True, impl=None):
         """MPNN.forward on the current observations (mpnn.py:40-77) -> (Q fp32 [B, N], argmax int32 [B])."""
         q = torch.zeros(self.B, self.NP, dtype=torch.float32, device=self.device)
         acts = self._actions if want_actions else None
         nm = float(norm_max) if norm_max is not None else 0.0
         if self.sparse:
-            if (self.mpnn_impl if impl is None else impl) == _lib.MPNN_TCGEN05:
-                raise NotImplementedError("the tensor-core MPNN needs the dense layout; sparse graph sets run the CUDA-core "
-                                          "gather forward")
+            use = self._sparse_impl(weights, impl)
             with torch.cuda.device(self.device):
-                check(lib().eco_smpnn_forward(C.byref(self.gs.c), C.byref(weights.c), self.B, _ptr(self.graph_idx),
-                                              _ptr(self.xn), _ptr(self.xg), nm, _ptr(q), _ptr(acts),
-                                              _ptr(self._scratch_for(self.B)), _stream()))
+                if use == _lib.MPNN_TCGEN05:
+                    check(lib().eco_smpnn_forward_impl(C.byref(self.gs.c), C.byref(weights.c), self.B, _ptr(self.graph_idx),
+                                                       _ptr(self.xn), _ptr(self.xg), nm, _ptr(q), _ptr(acts),
+                                                       _ptr(self._scratch_for(self.B)), use, _stream()))
+                else:
+                    check(lib().eco_smpnn_forward(C.byref(self.gs.c), C.byref(weights.c), self.B, _ptr(self.graph_idx),
+                                                  _ptr(self.xn), _ptr(self.xg), nm, _ptr(q), _ptr(acts),
+                                                  _ptr(self._scratch_for(self.B)), _stream()))
             return q[:, :self.N], acts
         forward = lib().eco_wmpnn_forward if self.weighted else lib().eco_mpnn_forward
         with torch.cuda.device(self.device):
@@ -668,12 +679,18 @@ class BatchedSpinSystem:
             raise ValueError("network policy needs weights")
         nm = float(norm_max) if norm_max is not None else -1.0
         if self.sparse:
+            use = self._sparse_impl(weights, impl) if pol == _lib.POLICY_NETWORK else _lib.MPNN_AUTO
             with torch.cuda.device(self.device):
-                check(lib().eco_srollout(C.byref(self.gs.c), C.byref(self.c),
-                                         C.byref(weights.c) if weights is not None else None, n_steps, pol, nm,
-                                         _ptr(self._actions),
-                                         _ptr(self._scratch_for(self.B)) if pol == _lib.POLICY_NETWORK else None,
-                                         _ptr(hist[0]), _ptr(hist[1]), _ptr(hist[2]), _stream()))
+                if use == _lib.MPNN_TCGEN05:
+                    check(lib().eco_srollout_impl(C.byref(self.gs.c), C.byref(self.c), C.byref(weights.c), n_steps, pol, nm,
+                                                  _ptr(self._actions), _ptr(self._scratch_for(self.B)), use,
+                                                  _ptr(hist[0]), _ptr(hist[1]), _ptr(hist[2]), _stream()))
+                else:
+                    check(lib().eco_srollout(C.byref(self.gs.c), C.byref(self.c),
+                                             C.byref(weights.c) if weights is not None else None, n_steps, pol, nm,
+                                             _ptr(self._actions),
+                                             _ptr(self._scratch_for(self.B)) if pol == _lib.POLICY_NETWORK else None,
+                                             _ptr(hist[0]), _ptr(hist[1]), _ptr(hist[2]), _stream()))
             self.current_step += n_steps
             return hist if record_history else None
         rollout = lib().eco_wrollout if self.weighted else lib().eco_rollout

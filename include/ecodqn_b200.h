@@ -484,6 +484,27 @@ int    eco_srollout(const eco_sgraphs_t* g, eco_env_t* env, const eco_mpnn_t* w,
                     float norm_max, int32_t* actions_scratch_dev, void* mpnn_scratch_dev, int32_t* hist_actions_dev,
                     double* hist_rewards_dev, double* hist_scores_dev, void* stream);
 
+/* The same two entries with a choice of Q-network implementation (MPNN.forward, reference src/networks/mpnn.py:40-159):
+ *   ECO_MPNN_AUTO, ECO_MPNN_SIMT  the gather forward above, fp32 CUDA cores; bit-identical to eco_smpnn_forward /
+ *                                 eco_srollout.
+ *   ECO_MPNN_TCGEN05              the same gathers, input stage and readout, with the seven per-vertex linears
+ *                                 (W_ef, and W_m, W_u of the three layers) on the tcgen05 tensor cores.  Needs
+ *                                 w->packed (eco_mpnn_pack output) and a 32-byte aligned scratch.  Serves every int8 CSR
+ *                                 set: the linears never read the couplings.
+ * Hi/lo operand rule of the tensor-core linears: every weight and every input activation x is split as x = hi + lo with
+ * hi = bf16(x), lo = bf16(x - hi); the product is W_hi x_hi + W_lo x_hi + W_hi x_lo with fp32 accumulation (W_lo x_lo is
+ * never formed), then fp32 ReLU.  Precision contract: per episode |q - q_fp64| <= 8e-4 * max_i |q_fp64_i| against the
+ * float64 forward, and |q - q_gather| <= 1e-3 |q| + 1e-4 max_i |q_i| against the gather forward (DESIGN.md section 2).
+ * Two calls on the same inputs give bit-identical Q, and an episode's Q does not depend on the other episodes of the
+ * batch.  An unknown impl, TCGEN05 without packed weights, a misaligned scratch and NULL pointers return
+ * ECO_ERR_INVALID before any launch.  Scratch sizes: eco_smpnn_scratch_bytes for every impl. */
+int    eco_smpnn_forward_impl(const eco_sgraphs_t* g, const eco_mpnn_t* w, int32_t B, const int32_t* graph_idx_dev,
+                              const float* xn_dev, const float* xg_dev, float norm_max, float* q_dev, int32_t* actions_dev,
+                              void* scratch_dev, int32_t impl, void* stream);
+int    eco_srollout_impl(const eco_sgraphs_t* g, eco_env_t* env, const eco_mpnn_t* w, int32_t n_steps, int32_t policy,
+                         float norm_max, int32_t* actions_scratch_dev, void* mpnn_scratch_dev, int32_t impl,
+                         int32_t* hist_actions_dev, double* hist_rewards_dev, double* hist_scores_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
